@@ -2,7 +2,7 @@
 """bench.py -- contact evals/sec (wrench + 6x6 Jacobians, FP64) of the batched
 ContinuousContactModel evaluation at 1/2/4/8 B200, with roofline, CPU baseline and end-to-end numbers.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A step = one pass of the hot path over one batch of synthetic contact states.
@@ -22,7 +22,8 @@ arg-min, strong), configs[2] (sampling-MPC batch 2 x 4096 x 100 per GPU, weak: p
 MPC step, fused integrate->contact->cost rollout), the rows next to the path, `e2e` through
 blf_ccm_eval_batch_host with HOST buffers, `cpu_baseline`, `sustained` (>= 1 s back to back).
 
-Prints ONE JSON line on rank 0.
+Prints ONE JSON line on rank 0.  --dump-outputs DIR also writes what the headline's last timed step
+handed its caller as .npy files (dump_outputs), so that two builds can be compared output for output.
 """
 from __future__ import annotations
 
@@ -50,6 +51,7 @@ BYTES_FULL_UNIFORM, BYTES_FULL_HET = 600, 632  # BASELINE.md section 3
 METRIC = "contact evals/sec (wrench+6x6 Jacobians, FP64)"
 UNIT = "evals/s"
 REF_WRENCH, WEIGHTS = [0.0, 0.0, 30.0, 0.0, 0.0, 0.0], [1.0, 10.0]
+DUMP_STATES = 1 << 16                         # --dump-outputs: states of the fixed, seeded output sample
 
 _JSON_OUT = None
 
@@ -197,7 +199,7 @@ def run_reference(args):
     impl, kind, what = _cpu_impl()
     for _ in range(max(1, min(args.warmup, 3))):
         impl.eval_batch_states(st, mask=7, nthreads=cores)
-    steps = max(1, min(args.steps, 50))  # bounded: each step is one 819 200-state pass
+    steps = max(1, args.steps)  # each step is one 819 200-state pass
     t0 = time.perf_counter()
     for _ in range(steps):
         impl.eval_batch_states(st, mask=7, nthreads=cores)
@@ -214,11 +216,11 @@ def run_reference(args):
         "cpu_baseline": {"value": value, "unit": UNIT, "cores": cores, "kind": kind,
                          "sample": sample},
         "e2e": {"value": value, "unit": UNIT, "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
-        "note": ("the reference's own sources, compiled from /root/reference into oracle/_ref against stand-in "
+        "note": ("the reference's own sources, compiled from BLF_REFERENCE_ROOT into oracle/_ref against stand-in "
                  "Eigen/iDynTree headers (the real libraries are absent from the image); a CPU rate does not "
                  "depend on the batch size, so each step times a bounded sample of the 2^28-state workload"
                  if kind == "reference"
-                 else "oracle/_ref was not built (no /root/reference at build time): C port timed"),
+                 else "oracle/_ref was not built (no BLF_REFERENCE_ROOT at build time): C port timed"),
     }
     if kind == "reference":  # the leaner C restatement beside it, for scale
         v, passes, spent, _, pwhat = cpu_reference_pass(st, cores, 2.0, prefer_reference=False)
@@ -310,7 +312,7 @@ class Ctx:
 
 def rollout_workload(cx: Ctx, what: str, total_rollouts: int, rollout_len: int, het: bool, K: int, W: int,
                      seed: int, sustain_s: float = 0.0, nsets: int = 1, host_planes=None,
-                     force_windows: int = 0) -> dict:
+                     force_windows: int = 0, dump_dir: str | None = None) -> dict:
     """One sharded sampling-MPC evaluation workload, timed as the contract says.
 
     Rank r owns rollouts [first, first+count) of `total_rollouts`.  A step = one
@@ -434,6 +436,10 @@ def rollout_workload(cx: Ctx, what: str, total_rollouts: int, rollout_len: int, 
     my_ms = e0.elapsed_time(e1)
     ms = cx.max_over_ranks(my_ms)
     clocks = cx.sampler.summary(t_host0, t_host1)
+    if dump_dir is not None and rank == 0:
+        last = W + K - 1
+        dump_outputs(dump_dir, torch, batch, bound[last % nsets][-1][1][2], sets[last % nsets][3],
+                     hist_g[last] if world > 1 else hist_l[last])
 
     # ---- blocked-peer probe: the last rank arrives 50 ms late, four times; nobody may mix epochs
     probe_steps = 4 if world > 1 else 0
@@ -561,6 +567,24 @@ def rollout_workload(cx: Ctx, what: str, total_rollouts: int, rollout_len: int, 
            "clocks": clocks, "parity": parity, "exchange_check": exchange_check, "collective": cx.collective_name(),
            "argmin": {"cost": bc, "rollout": bi}, "sustained": sustained}
     return res
+
+
+def dump_outputs(out_dir: str, torch, batch, out: dict, cost, best_pair) -> None:
+    """What one step of blf_ccm_rollout_cost_argmin_soa handed its caller, as float64 .npy files: the
+    wrench, autonomous dynamics and control matrix of a fixed, seeded sample of the states (indices in
+    state_index; within the last output window when the outputs are windowed), every rollout's cost and
+    the arg-min pair (best = [cost, rollout]).  About 34 MB for the headline on one GPU."""
+    torch.cuda.synchronize()
+    n = out["ctrl"].shape[0]
+    idx_np = np.unique(np.random.default_rng(2024).integers(0, n, DUMP_STATES))
+    idx = torch.from_numpy(idx_np).to(out["ctrl"].device)
+    bc, bi = batch.decode_best(best_pair)
+    arrays = {"state_index": idx_np, "wrench": out["wrench"][:, idx].T, "autodyn": out["autodyn"][:, idx].T,
+              "ctrl": out["ctrl"][idx], "cost": cost, "best": np.array([bc, bi])}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        a = a.cpu().numpy() if hasattr(a, "cpu") else a
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a, dtype=np.float64))
 
 
 def eval_only_leg(cx: Ctx, planes_np, K: int, W: int) -> dict:
@@ -872,7 +896,7 @@ def run_ours(args):
 
     head = rollout_workload(
         cx, "configs[4]", HEAD_ROLLOUTS, HEAD_ROLLOUT_LEN, het=False, K=K, W=W, seed=46,
-        sustain_s=0.0 if args.only_main else 1.2, force_windows=args.force_windows)
+        sustain_s=0.0 if args.only_main else 1.2, force_windows=args.force_windows, dump_dir=args.dump_outputs)
     line = {
         "metric": METRIC, "value": head["value"], "unit": UNIT, "n_gpus": cx.world, "steps": K, "warmup": W,
         "ms_per_step": head["ms_per_step"], "higher_is_better": True, "scaling": "strong",
@@ -952,7 +976,7 @@ def run_config2(args):
     cx = Ctx(args)
     torch, syn, batch, dev = cx.torch, cx.syn, cx.batch, cx.dev
     n, nsets = 1 << 20, 3
-    K, W = min(args.steps, 2000), max(min(args.warmup, 10), 3)
+    K, W = max(1, args.steps), max(min(args.warmup, 10), 3)
     planes, _ = syn.make_planes_torch(n, dev, seed=43 + 1000 * cx.rank)
     sets = [(planes, batch.alloc_soa_outputs(n, WRENCH))] + \
         [([None if q is None else q.clone() for q in planes], batch.alloc_soa_outputs(n, WRENCH))
@@ -1019,7 +1043,11 @@ def main():
                     help="profiling aid: run only the headline timed loop (no extra records)")
     ap.add_argument("--force-windows", type=int, default=0,
                     help="testing aid: reuse an output window of 1/W of the shard (the low-memory fallback)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="headline workload: write what the last timed step computed to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs is not None and (args.impl != "ours" or args.workload != "headline"):
+        ap.error("--dump-outputs applies to the headline workload of --impl ours")
     # stdout carries exactly ONE JSON line: whatever libraries print there (NCCL's version banner
     # when NCCL_DEBUG is set on the box) is sent to stderr at the file-descriptor level
     global _JSON_OUT

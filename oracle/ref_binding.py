@@ -7,9 +7,9 @@ What the library is (oracle/refbuild/README.md): the unmodified translation unit
 src/ContactModels/src/{ContactModel,ContinuousContactModel}.cpp,
 src/ParametersHandler/src/StdImplementation.cpp, src/Estimators/src/RecursiveLeastSquare.cpp,
 src/System/src/FloatingBaseSystemKinematics.cpp (+ the header-only ForwardEuler / FixedStepIntegrator)
-compiled from /root/reference against stand-in Eigen / iDynTree headers, plus
-oracle/refbuild/ref_driver.cpp, which only calls their public interface.  It can be (re)built only
-where /root/reference exists; the built .so travels to the GPU box with the snapshot.
+compiled from the original project's tree named by BLF_REFERENCE_ROOT against stand-in Eigen /
+iDynTree headers, plus oracle/refbuild/ref_driver.cpp, which only calls their public interface.  It
+can be (re)built only where that tree is given; tests/reference_samples.py stands in for it elsewhere.
 """
 from __future__ import annotations
 
@@ -23,7 +23,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 REF_DIR = os.path.join(_HERE, "_ref")
 LIB_PATH = os.path.join(REF_DIR, "libblf_reference.so")
 REFBUILD_DIR = os.path.join(_HERE, "refbuild")
-REFERENCE_ROOT = os.environ.get("BLF_REFERENCE_ROOT", "/root/reference")
+REFERENCE_ROOT = os.environ.get("BLF_REFERENCE_ROOT", "")   # the original project's source tree, when given
 REFERENCE_TESTS = ("ContinuousContactModelReferenceTests", "IntegratorReferenceTests",
                    "ParametersHandlerReferenceTests")
 FACADE_TEST = "ContinuousContactModelReferenceTests_on_b200_facade"  # needs a CUDA device to run
@@ -34,22 +34,24 @@ WRENCH, AUTODYN, CTRL, REGRESSOR = 1, 2, 4, 8
 
 
 def reference_sources_present() -> bool:
-    return os.path.isfile(os.path.join(REFERENCE_ROOT, "src", "ContactModels", "src",
-                                       "ContinuousContactModel.cpp"))
+    return bool(REFERENCE_ROOT) and os.path.isfile(
+        os.path.join(REFERENCE_ROOT, "src", "ContactModels", "src", "ContinuousContactModel.cpp"))
 
 
 def build(force: bool = False) -> str | None:
-    """make -C oracle/refbuild (needs the reference tree).  Returns the library path, or None when
-    the reference tree is absent and nothing was prebuilt."""
+    """make -C oracle/refbuild: the stand-in self-test and the facade driver always, the reference
+    build where the reference tree is given.  Returns the reference library's path, or None when the
+    reference tree is absent and nothing was prebuilt."""
+    facade = os.path.exists(os.path.join(os.path.dirname(_HERE), "bipedal_locomotion_framework_b200", "lib",
+                                         "libblf_contact.so"))
+    targets = ["selftest"] + (["facade_driver"] if facade else [])
     if reference_sources_present():
-        targets = ["all"]
-        if os.path.exists(os.path.join(os.path.dirname(_HERE), "bipedal_locomotion_framework_b200", "lib",
-                                       "libblf_contact.so")):
-            targets.append("facade")  # the reference's unmodified test linked to the product facade
-        cmd = ["make", "-C", REFBUILD_DIR, f"REF={REFERENCE_ROOT}", *targets] + (["-B"] if force else [])
-        r = subprocess.run(cmd, stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True)
-        if r.returncode != 0:
-            raise RuntimeError("building oracle/_ref failed:\n" + r.stdout)
+        # + the reference's unmodified tests linked to the product facade
+        targets = ["all"] + (["facade"] if facade else [])
+    cmd = ["make", "-C", REFBUILD_DIR, f"REF={REFERENCE_ROOT}", *targets] + (["-B"] if force else [])
+    r = subprocess.run(cmd, stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True)
+    if r.returncode != 0:
+        raise RuntimeError("building oracle/_ref failed:\n" + r.stdout)
     return LIB_PATH if os.path.exists(LIB_PATH) else None
 
 
@@ -76,8 +78,8 @@ def lib():
     global _lib
     if _lib is None:
         if not os.path.exists(LIB_PATH) and build() is None:
-            raise RuntimeError("oracle/_ref/libblf_reference.so is absent and /root/reference is not "
-                               "here to build it from")
+            raise RuntimeError("oracle/_ref/libblf_reference.so is absent and BLF_REFERENCE_ROOT names no "
+                               "reference tree to build it from")
         L = C.CDLL(LIB_PATH)
         vp, d, i, sz = C.c_void_p, C.c_double, C.c_int, C.c_size_t
         L.blf_ref_description.restype = C.c_char_p

@@ -1,7 +1,7 @@
 """CPU tests that PIN THE ORACLE AGAINST THE REFERENCE'S OWN SOURCES (no GPU).
 
-oracle/_ref/libblf_reference.so is the reference's unmodified .cpp files compiled from /root/reference
-against stand-in Eigen/iDynTree headers (oracle/refbuild/).  Here:
+oracle/_ref/libblf_reference.so is the reference's unmodified .cpp files compiled from the original
+project's tree named by BLF_REFERENCE_ROOT against stand-in Eigen/iDynTree headers (oracle/refbuild/).  Here:
   * the reference's own Catch2 tests (ContinousContactModelTest.cpp, IntegratorTest.cpp,
     ParametersHandlerTest.cpp), compiled unmodified, pass on that build -- which validates the
     stand-in headers through the reference's own properties (Monte-Carlo integral, regressor
@@ -10,7 +10,7 @@ against stand-in Eigen/iDynTree headers (oracle/refbuild/).  Here:
     follow the same expression structure and agree BIT FOR BIT, which the tests require;
   * the reference build is compared with the exact-rational golden vectors;
   * the reference's error / lazy-cache behaviour is observed and pinned.
-The tests skip (not fail) where neither /root/reference nor a prebuilt oracle/_ref exists.
+The tests skip (not fail) where neither that tree nor a prebuilt oracle/_ref exists.
 """
 import json
 import os
@@ -30,7 +30,7 @@ DEGENERATE_ROW = 8
 def ref():
     from oracle import ref_binding
     if not ref_binding.available():
-        pytest.skip("oracle/_ref is not built and /root/reference is not present to build it")
+        pytest.skip("oracle/_ref is not built and BLF_REFERENCE_ROOT names no reference tree to build it from")
     ref_binding.build()  # refresh when the reference tree is here (make is incremental)
     return ref_binding
 
