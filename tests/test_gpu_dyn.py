@@ -459,6 +459,17 @@ def test_facade_class_vs_reference_class(torch, ref, cps, ncols, het, with_reg):
         assert rel(fq, rq).max() <= TOL
 
 
+def _place(torch, a, shift):
+    """`a` on the device, `shift` doubles into a fresh buffer: 16-byte aligned (0) or 8 bytes off (1)."""
+    if a is None:
+        return None
+    buf = torch.empty(a.size + 2, dtype=torch.float64, device="cuda")
+    v = buf[shift:shift + a.size].view(a.shape)
+    v.copy_(torch.from_numpy(np.ascontiguousarray(a)))
+    assert v.data_ptr() % 16 == 8 * shift
+    return v
+
+
 @pytest.mark.parametrize("nc,ns,with_reg", [(6, 4_099, False), (8, 2_051, True), (12, 4_099, False), (12, 1_003, True),
                                             (12, 5, False), (6, 1, False), (10, 3_001, True), (14, 2_003, False)])
 def test_mass_matrix_solve_bulk_and_per_thread_fill_agree(torch, dyn, so, nc, ns, with_reg):
@@ -469,15 +480,7 @@ def test_mass_matrix_solve_bulk_and_per_thread_fill_agree(torch, dyn, so, nc, ns
     want = so.mass_matrix_solve(M, known, tau, reg, nthreads=NTHREADS)
 
     def run(shift):
-        def place(a):   # the array `shift` doubles into a fresh buffer: 16-byte aligned (0) or 8 bytes off (1)
-            if a is None:
-                return None
-            buf = torch.empty(a.size + 2, dtype=torch.float64, device="cuda")
-            v = buf[shift:shift + a.size].view(a.shape)
-            v.copy_(torch.from_numpy(np.ascontiguousarray(a)))
-            assert v.data_ptr() % 16 == 8 * shift
-            return v
-        dM, dk, dt = place(M), place(known), place(tau)
+        dM, dk, dt = (_place(torch, a, shift) for a in (M, known, tau))
         x = dyn.solve(dM, dk, dt, _dev(torch, reg)).cpu().numpy()
         dyn.solve(dM, dk, dt, _dev(torch, reg), out=dk)          # in place: acc may alias known
         assert np.array_equal(dk.cpu().numpy(), x)
@@ -486,3 +489,123 @@ def test_mass_matrix_solve_bulk_and_per_thread_fill_agree(torch, dyn, so, nc, ns
     bulk, per_thread = run(0), run(1)
     assert np.array_equal(bulk, per_thread)
     assert rel(bulk, want).max() <= TOL
+
+
+# --- batches the solve's persistent warps take in several passes -----------------------------------------
+
+def _multi_pass(torch, nc):
+    """(ns, W, SPW) for a batch that every warp of the warp-level solve takes in three passes or more.
+    A warp solves SPW systems at a time (8 up to 15 unknowns, 4 up to 31, 2 up to 47, 1 up to 64: the lane
+    classes of csrc/dyn_kernels.cu) and strides over the groups of SPW by the number of warps launched.
+    The launcher caps the grid at the CTAs of 64 threads that are resident at once, so no launch has more
+    than W = SMs x max threads per SM / 32 warps, whatever the occupancy, and 3 W SPW systems need three
+    passes.  The extra 37 SPW + (SPW + 1) // 2 systems make the last group ragged (SPW > 1) and the group
+    count 3 W + 38, no multiple of W.  148-SM B200: 227 k systems up to 15 unknowns, 114 k up to 31,
+    57 k up to 47, 28 k up to 64."""
+    p = torch.cuda.get_device_properties(0)
+    spw = 8 if nc <= 15 else 4 if nc <= 31 else 2 if nc <= 47 else 1
+    w = p.multi_processor_count * p.max_threads_per_multi_processor // 32
+    return 3 * w * spw + 37 * spw + (spw + 1) // 2, w, spw
+
+
+BULK_ORDERS = (6, 8, 10, 12, 14)   # even orders that fill a 4-lane class exactly: the bulk-copy fill when aligned
+MULTI_PASS_ORDERS = BULK_ORDERS + (5, 9, 15) + (16, 23, 24, 29, 31) + (32, 38, 47) + (48, 59, 64)
+
+
+@pytest.mark.parametrize("nc,with_reg", [(nc, i % 2 == 1) for i, nc in enumerate(MULTI_PASS_ORDERS)])
+def test_mass_matrix_solve_multi_pass_vs_oracle(torch, batch, dyn, so, nc, with_reg):
+    """Every lane class (4, 8, 16, 32 lanes per system; 24 unknowns: the right-hand side as a column) on a
+    batch its warps take in three passes or more, so the tiles are refilled for the next group while the
+    current one is factorised: within 1e-12 of the oracle, nothing written outside the output, in place =
+    out of place bit for bit.  The even orders up to 14 run twice, 16-byte aligned (bulk-copy refills on the
+    warp's mbarrier) and 8 bytes off (per-thread copies): bit-identical."""
+    ns = _multi_pass(torch, nc)[0]
+    M, known, tau, reg = _case(nc, ns, 1300 + nc, with_reg=with_reg)
+    want = so.mass_matrix_solve(M, known, tau, reg, nthreads=NTHREADS)
+    dr = _dev(torch, reg)
+
+    def run(shift):
+        dM, dk, dt = (_place(torch, a, shift) for a in (M, known, tau))
+        guard = torch.full((ns + 2, nc), 123.0, dtype=torch.float64, device="cuda")
+        x = dyn.solve(dM, dk, dt, dr, out=guard[1:ns + 1])
+        assert _last_path(batch) == PATH_LLT_WARP
+        assert bool((guard[0] == 123.0).all()) and bool((guard[ns + 1] == 123.0).all())   # nothing written outside
+        dyn.solve(dM, dk, dt, dr, out=dk)          # in place, as the whole step solves
+        assert torch.equal(dk, x)
+        return x.cpu().numpy()
+
+    x = run(0)
+    assert np.isfinite(x).all()
+    err = rel(x, want)
+    assert err.max() <= TOL, (ns, int(np.argmax(err)), err.max())
+    if nc in BULK_ORDERS:
+        y = run(1)
+        assert np.array_equal(y, x), (ns, int(np.argmax(np.abs(y - x).max(axis=1))))
+
+
+@pytest.mark.parametrize("nc", [12, 14, 15, 29, 38])
+def test_mass_matrix_solve_position_invariant_across_passes(torch, dyn, nc):
+    """A system's arithmetic does not depend on where it sits in the batch: the systems of a multi-pass batch
+    equal, bit for bit, the same systems solved as a batch of their own that takes one pass -- the first
+    ones, the ones from W SPW on (no earlier than the second pass) and the ragged tail.  Catches a refill of
+    the wrong group or a stale tile even where its error would fit inside 1e-12.  Slices of even orders
+    stay 16-byte aligned: 12 and 14 take the bulk-copy fill in both calls."""
+    ns, w, spw = _multi_pass(torch, nc)
+    M, known, tau, reg = _case(nc, ns, 1400 + nc, with_reg=True)
+    dM, dk, dt, dr = (_dev(torch, a) for a in (M, known, tau, reg))
+    x = dyn.solve(dM, dk, dt, dr)
+    # 2 x SMs groups: a warp per group, one pass, since at least one CTA of two warps per SM is resident
+    c = 2 * torch.cuda.get_device_properties(0).multi_processor_count * spw - 1
+    for a in (0, w * spw, ns - c):
+        part = dyn.solve(dM[a:a + c], dk[a:a + c], None if dt is None else dt[a:a + c], dr)
+        assert torch.equal(part, x[a:a + c]), (ns, a)
+
+
+@pytest.mark.parametrize("nc", [12, 38])
+def test_not_positive_definite_stays_local_across_passes(torch, dyn, nc):
+    """Systems that are not positive definite in the first pass, in a later one and in the ragged last group
+    give NaN; every other system is bit-identical to the batch without them.  38 unknowns (16-lane groups,
+    blocked back substitution) read entries of the diagonal-block buffer that only earlier passes wrote --
+    NaN after a bad system -- into lanes that hold no unknown: harmless, and pinned here."""
+    ns, w, spw = _multi_pass(torch, nc)
+    M, known, tau, reg = _case(nc, ns, 1500 + nc, with_reg=True)
+    dk, dt, dr = (_dev(torch, a) for a in (known, tau, reg))
+    x0 = dyn.solve(_dev(torch, M), dk, dt, dr).cpu().numpy()
+    bad = [3, 2 * w * spw + 5, ns - 1]
+    M[bad[0]] = -M[bad[0]]
+    M[bad[1], 5, 5] = -1.0
+    M[bad[2], nc - 1, nc - 1] = -1.0
+    x1 = dyn.solve(_dev(torch, M), dk, dt, dr).cpu().numpy()
+    assert np.array_equal(np.flatnonzero(np.isnan(x1).any(axis=1)), bad), ns
+    ok = np.ones(ns, dtype=bool)
+    ok[bad] = False
+    assert np.array_equal(x1[ok], x0[ok]), ns
+
+
+@pytest.mark.parametrize("ncols,het,with_reg", [(12, False, True), (6, True, False)])
+def test_floating_base_acceleration_multi_pass_vs_oracle(torch, batch, dyn, so, ncols, het, with_reg):
+    """blf_sys_floating_base_acceleration at the small sizes of the benchmark, 2 contacts, on a batch whose
+    solve takes three passes or more: the solve runs in place on the bulk-copy fill.  Against the C oracle
+    within the conditioning-aware bound of the whole step."""
+    cps = 2
+    ns = _multi_pass(torch, ncols)[0]
+    n = ns * cps
+    st = syn.make_states(n, seed=160 + ncols, heterogeneous=het)
+    rng = np.random.default_rng(161 + ncols)
+    J = rng.uniform(-1.0, 1.0, (n, 6, ncols))
+    bias = rng.uniform(-50.0, 50.0, (ns, ncols))
+    M, _, tau, reg = _case(ncols, ns, 162 + ncols, with_reg=with_reg)
+    planes = syn.aos_to_planes(st["twists"], st["poses"], st["null_poses"])
+    prm = st["params"].T if het else None
+    want, wr = so.floating_base_acceleration(cps, planes, J, bias, M, tau, reg, param_planes=prm,
+                                             uniform=syn.REFERENCE_TEST_PARAMS, want_wrench=True, nthreads=NTHREADS)
+    acc = dyn.acceleration(cps, _dev(torch, planes), _dev(torch, J), _dev(torch, bias), _dev(torch, M),
+                           _dev(torch, tau), _dev(torch, reg), param_planes=_dev(torch, prm))
+    assert _last_path(batch) == PATH_LLT_WARP
+    mag = np.abs(bias) + np.einsum("scrq,scr->sq", np.abs(J.reshape(ns, cps, 6, ncols)),
+                                   np.abs(wr.T.reshape(ns, cps, 6)))
+    if tau is not None:
+        mag[:, 6:] += np.abs(tau)
+    tol = _acc_tolerance(M if reg is None else M + reg, want, mag.max(axis=1))
+    err = np.abs(acc.cpu().numpy() - want).max(axis=1)
+    assert (err <= tol).all(), (ns, int(np.argmax(err / tol)), (err / tol).max())
