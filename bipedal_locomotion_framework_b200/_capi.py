@@ -23,7 +23,8 @@ SYMBOLS = [
     "blf_ccm_eval_surface_points",
     "blf_ccm_rollout_cost_argmin_soa", "blf_ccm_argmin_pairs", "blf_ccm_argmin_allgather_nccl",
     "blf_ccm_last_path", "blf_ccm_launch_count", "blf_ccm_device", "blf_ccm_sm_count",
-    "blf_ccm_device_alloc", "blf_ccm_device_free", "blf_ccm_host_alloc", "blf_ccm_host_free",
+    "blf_ccm_device_alloc", "blf_ccm_device_free", "blf_ccm_device_alloc_compressible",
+    "blf_ccm_pointer_is_compressible", "blf_ccm_host_alloc", "blf_ccm_host_free",
     "blf_ccm_copy_h2d", "blf_ccm_copy_d2h", "blf_ccm_stream_synchronize",
     "blf_rls_advance_batch", "blf_rls_advance_host", "blf_ccm_rls_advance_contacts",
     "blf_sys_kinematics_euler_step_soa", "blf_sys_kinematics_dynamics_host", "blf_sys_kinematics_dynamics",
@@ -72,6 +73,8 @@ def lib():
     u64 = C.c_uint64
     L.blf_ccm_device_alloc.argtypes = [vp, u64, C.POINTER(vp)]
     L.blf_ccm_device_free.argtypes = [vp, vp]
+    L.blf_ccm_device_alloc_compressible.argtypes = [vp, u64, C.POINTER(vp), C.POINTER(ci)]
+    L.blf_ccm_pointer_is_compressible.argtypes = [vp, vp, C.POINTER(ci)]
     L.blf_ccm_host_alloc.argtypes = [vp, u64, C.POINTER(vp)]
     L.blf_ccm_host_free.argtypes = [vp, vp]
     L.blf_ccm_copy_h2d.argtypes = [vp, vp, vp, u64, vp]

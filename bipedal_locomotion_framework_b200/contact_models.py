@@ -12,6 +12,7 @@ pytest / bench harness.  torch supplies device memory and streams (plumbing only
 from __future__ import annotations
 
 import ctypes as C
+import os
 import sys
 
 import numpy as np
@@ -130,6 +131,32 @@ class _Handle:
     @property
     def sm_count(self) -> int:
         return int(_capi.lib().blf_ccm_sm_count(self._h))
+
+
+class _CompressibleBuffer:
+    """Owner of one blf_ccm_device_alloc_compressible allocation of float64s, exposed through
+    __cuda_array_interface__.  A tensor made from it with torch.as_tensor holds a reference to it,
+    and so does every view or slice of that tensor: the memory is freed (after a device
+    synchronise, see blf_ccm_device_free) when the last of them goes away."""
+
+    def __init__(self, handle: _Handle, shape):
+        self._handle = handle            # the handle must outlive the allocation
+        self.ptr = 0
+        p, granted = C.c_void_p(), C.c_int()
+        _capi.check(_capi.lib().blf_ccm_device_alloc_compressible(
+            handle.ptr, 8 * int(np.prod(shape)), C.byref(p), C.byref(granted)))
+        self.ptr = p.value or 0
+        self.granted = bool(granted.value)
+        self.__cuda_array_interface__ = {"shape": tuple(shape), "typestr": "<f8", "data": (self.ptr, False),
+                                         "strides": None, "version": 3}
+
+    def __del__(self):
+        if self.ptr:
+            try:
+                _capi.lib().blf_ccm_device_free(self._handle.ptr, self.ptr)
+            except Exception:
+                pass
+            self.ptr = 0
 
 
 def _np_ptr(a):
@@ -329,13 +356,30 @@ class ContinuousContactModelBatch:
     def _stream(self):
         return self._torch.cuda.current_stream(self.device).cuda_stream
 
+    def alloc_ctrl(self, n: int):
+        """(n, 36) float64 device tensor for the dense control matrix, in compressible memory where
+        the device supports it (blf_ccm_device_alloc_compressible): 24 of the 36 entries are
+        structural +0.0, so the hardware moves fewer bytes to and from HBM; the values are the
+        ones written.  BLF_CCM_TUNE_NO_COMPRESS=1 gives a plain torch.empty tensor."""
+        t = self._torch
+        if n == 0 or os.environ.get("BLF_CCM_TUNE_NO_COMPRESS", "0") not in ("", "0"):
+            return t.empty((n, 36), dtype=t.float64, device=self.device)
+        return t.as_tensor(_CompressibleBuffer(self._handle, (n, 36)), device=self.device)
+
+    def is_compressible(self, tensor) -> bool:
+        """True when the tensor's memory lies in a compressible allocation of this batch's handle."""
+        out = C.c_int()
+        _capi.check(_capi.lib().blf_ccm_pointer_is_compressible(self._handle.ptr, tensor.data_ptr(),
+                                                                C.byref(out)))
+        return bool(out.value)
+
     def alloc_soa_outputs(self, n: int, mask: int) -> dict:
         t = self._torch
         mk = lambda *s: t.empty(s, dtype=t.float64, device=self.device)
         return {
             "wrench": mk(6, n) if mask & WRENCH else None,
             "autodyn": mk(6, n) if mask & AUTODYN else None,
-            "ctrl": mk(n, 36) if mask & CTRL else None,
+            "ctrl": self.alloc_ctrl(n) if mask & CTRL else None,
             "regressor": mk(12, n) if mask & REGRESSOR else None,
         }
 
@@ -345,7 +389,7 @@ class ContinuousContactModelBatch:
         return {
             "wrench": mk(n, 6) if mask & WRENCH else None,
             "autodyn": mk(n, 6) if mask & AUTODYN else None,
-            "ctrl": mk(n, 36) if mask & CTRL else None,
+            "ctrl": self.alloc_ctrl(n) if mask & CTRL else None,
             "regressor": mk(n, 12) if mask & REGRESSOR else None,
         }
 

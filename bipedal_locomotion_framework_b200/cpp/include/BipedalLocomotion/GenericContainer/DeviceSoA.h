@@ -36,8 +36,12 @@ class DeviceSoA
 
 public:
     DeviceSoA() = default;
-    /** Owning container of `planes` x `size` doubles. */
-    DeviceSoA(std::shared_ptr<ContactModels::CudaDevice> device, std::size_t planes, std::size_t size);
+    /** Owning container of `planes` x `size` doubles.  `compressible`: request Compute Data
+     * Compression for the allocation (blf_ccm_device_alloc_compressible; plain memory where the
+     * device does not grant it), for data with many zeros such as the dense n x 36 control matrix
+     * (one plane of 36 n doubles). */
+    DeviceSoA(std::shared_ptr<ContactModels::CudaDevice> device, std::size_t planes, std::size_t size,
+              bool compressible = false);
     /** Non-owning view over existing device planes. */
     DeviceSoA(std::shared_ptr<ContactModels::CudaDevice> device, const std::vector<double*>& planes,
               std::size_t size);

@@ -2,6 +2,7 @@
  * @file DeviceSoA.cpp
  * Device-side structure-of-arrays container over the C ABI's memory helpers.
  */
+#include <cstdint>
 #include <iostream>
 #include <utility>
 #include <vector>
@@ -22,13 +23,17 @@ blf_ccm_handle* raw(const std::shared_ptr<CudaDevice>& d)
 }
 } // namespace
 
-DeviceSoA::DeviceSoA(std::shared_ptr<CudaDevice> device, std::size_t planes, std::size_t size)
+DeviceSoA::DeviceSoA(std::shared_ptr<CudaDevice> device, std::size_t planes, std::size_t size,
+                     bool compressible)
     : m_device(std::move(device)), m_size(size), m_owning(true)
 {
     if (m_device == nullptr || planes == 0) return;
     m_pitch = (size + 31) / 32 * 32; // planes start on 256-byte boundaries
     if (m_pitch == 0) m_pitch = 32;
-    if (blf_ccm_device_alloc(raw(m_device), planes * m_pitch * sizeof(double), &m_base) != BLF_CCM_OK)
+    const std::uint64_t bytes = planes * m_pitch * sizeof(double);
+    const int rc = compressible ? blf_ccm_device_alloc_compressible(raw(m_device), bytes, &m_base, nullptr)
+                                : blf_ccm_device_alloc(raw(m_device), bytes, &m_base);
+    if (rc != BLF_CCM_OK)
     {
         std::cerr << "[DeviceSoA::DeviceSoA] " << blf_ccm_last_error() << std::endl;
         m_base = nullptr;

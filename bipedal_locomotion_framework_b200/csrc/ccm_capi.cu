@@ -14,6 +14,7 @@
 #include <cstdlib>
 #include <cstring>
 #include <map>
+#include <mutex>
 #include <new>
 #include <type_traits>
 
@@ -68,6 +69,13 @@ struct TensorMapEntry {
     int horizon = 0;
     long long chains = 0;
     CUtensorMap map;
+};
+
+// one blf_ccm_device_alloc_compressible allocation: a reserved virtual range with one physical
+// compressible allocation mapped onto it
+struct VmmRange {
+    size_t size = 0;
+    CUmemGenericAllocationHandle mem = 0;
 };
 
 struct blf_ccm_handle {
@@ -136,6 +144,10 @@ struct blf_ccm_handle {
     P2pSlot* p2p_peer[kP2pMaxRanks] = {};     // every rank's mailbox as mapped here
     unsigned long long p2p_epoch = 0;
     CostIdx* p2p_fused_out = nullptr;         // non-NULL: rollout reductions also run the exchange
+    // compressible allocations by base address; every other device pointer is cudaMalloc memory.
+    // Locked: owners may free from another thread (e.g. a garbage collector).
+    std::map<uintptr_t, VmmRange> vmm;
+    std::mutex vmm_mutex;
 };
 
 static int env_int(const char* name)
@@ -192,6 +204,7 @@ struct NvtxRange {
 // path pays nothing.
 static int scratch_acquire(blf_ccm_handle* h, cudaStream_t st);
 static int scratch_quiesce(blf_ccm_handle* h);
+static void vmm_release_all(blf_ccm_handle* h);
 
 extern "C" const char* blf_ccm_version(void) { return "blf_ccm 0.1.0 (sm_100a)"; }
 extern "C" const char* blf_ccm_last_error(void) { return g_err; }
@@ -317,6 +330,7 @@ extern "C" int blf_ccm_destroy(blf_ccm_handle* h)
         if (h->hev_down[s]) cudaEventDestroy(h->hev_down[s]);
     }
     p2p_release(h);
+    vmm_release_all(h);
     if (h->single_out) cudaFreeHost(h->single_out);
     if (h->block_best) cudaFree(h->block_best);
     if (h->counter) cudaFree(h->counter);
@@ -1385,10 +1399,162 @@ extern "C" int blf_ccm_device_alloc(blf_ccm_handle* h, uint64_t bytes, void** ou
     return BLF_CCM_OK;
 }
 
+// Compute Data Compression is requested per allocation through the driver's virtual-memory calls
+// (cuMemCreate with CU_MEM_ALLOCATION_COMP_GENERIC).  The entry points are looked up once through
+// the runtime (no -lcuda), as cuTensorMapEncodeTiled is; ok is false when one of them is missing.
+struct VmmApi {
+    bool ok = false;
+    CUresult (*get_attribute)(int*, CUdevice_attribute, CUdevice) = nullptr;
+    CUresult (*granularity)(size_t*, const CUmemAllocationProp*, CUmemAllocationGranularity_flags) = nullptr;
+    CUresult (*create)(CUmemGenericAllocationHandle*, size_t, const CUmemAllocationProp*, unsigned long long) = nullptr;
+    CUresult (*properties)(CUmemAllocationProp*, CUmemGenericAllocationHandle) = nullptr;
+    CUresult (*reserve)(CUdeviceptr*, size_t, size_t, CUdeviceptr, unsigned long long) = nullptr;
+    CUresult (*map)(CUdeviceptr, size_t, size_t, CUmemGenericAllocationHandle, unsigned long long) = nullptr;
+    CUresult (*set_access)(CUdeviceptr, size_t, const CUmemAccessDesc*, size_t) = nullptr;
+    CUresult (*unmap)(CUdeviceptr, size_t) = nullptr;
+    CUresult (*address_free)(CUdeviceptr, size_t) = nullptr;
+    CUresult (*release)(CUmemGenericAllocationHandle) = nullptr;
+};
+
+static const VmmApi& vmm_api()
+{
+    static const VmmApi api = [] {
+        VmmApi a;
+        bool all = true;
+        auto get = [&all](const char* name, auto& fn) {
+            void* p = nullptr;
+            cudaDriverEntryPointQueryResult q;
+            if (cudaGetDriverEntryPoint(name, &p, cudaEnableDefault, &q) != cudaSuccess ||
+                q != cudaDriverEntryPointSuccess) {
+                cudaGetLastError();
+                p = nullptr;
+            }
+            fn = reinterpret_cast<std::remove_reference_t<decltype(fn)>>(p);
+            all = all && p != nullptr;
+        };
+        get("cuDeviceGetAttribute", a.get_attribute);
+        get("cuMemGetAllocationGranularity", a.granularity);
+        get("cuMemCreate", a.create);
+        get("cuMemGetAllocationPropertiesFromHandle", a.properties);
+        get("cuMemAddressReserve", a.reserve);
+        get("cuMemMap", a.map);
+        get("cuMemSetAccess", a.set_access);
+        get("cuMemUnmap", a.unmap);
+        get("cuMemAddressFree", a.address_free);
+        get("cuMemRelease", a.release);
+        a.ok = all;
+        return a;
+    }();
+    return api;
+}
+
+// A compressible mapping of `bytes` on the handle's device, or false (nothing held) when the device
+// has no compression, the driver does not grant it for this allocation, or any step fails.
+static bool vmm_map_compressible(blf_ccm_handle* h, uint64_t bytes, void** out)
+{
+    const VmmApi& api = vmm_api();
+    int supported = 0;
+    if (!api.ok ||
+        api.get_attribute(&supported, CU_DEVICE_ATTRIBUTE_GENERIC_COMPRESSION_SUPPORTED, h->device) != CUDA_SUCCESS ||
+        !supported)
+        return false;
+    CUmemAllocationProp prop = {};
+    prop.type = CU_MEM_ALLOCATION_TYPE_PINNED;
+    prop.location.type = CU_MEM_LOCATION_TYPE_DEVICE;
+    prop.location.id = h->device;
+    prop.allocFlags.compressionType = CU_MEM_ALLOCATION_COMP_GENERIC;
+    size_t gran = 0;
+    if (api.granularity(&gran, &prop, CU_MEM_ALLOC_GRANULARITY_RECOMMENDED) != CUDA_SUCCESS || gran == 0)
+        return false;
+    const size_t size = (bytes + gran - 1) / gran * gran;
+    CUmemGenericAllocationHandle mem = 0;
+    if (api.create(&mem, size, &prop, 0) != CUDA_SUCCESS) return false;
+    // the driver may drop the request silently: only what it reports as granted counts
+    CUmemAllocationProp got = {};
+    bool ok = api.properties(&got, mem) == CUDA_SUCCESS &&
+              got.allocFlags.compressionType == CU_MEM_ALLOCATION_COMP_GENERIC;
+    CUdeviceptr base = 0;
+    ok = ok && api.reserve(&base, size, gran, 0, 0) == CUDA_SUCCESS;
+    bool mapped = ok && api.map(base, size, 0, mem, 0) == CUDA_SUCCESS;
+    CUmemAccessDesc access = {};
+    access.location = prop.location;
+    access.flags = CU_MEM_ACCESS_FLAGS_PROT_READWRITE;
+    ok = mapped && api.set_access(base, size, &access, 1) == CUDA_SUCCESS;
+    if (!ok) {
+        if (mapped) api.unmap(base, size);
+        if (base) api.address_free(base, size);
+        api.release(mem);
+        return false;
+    }
+    {
+        std::lock_guard<std::mutex> lock(h->vmm_mutex);
+        h->vmm[static_cast<uintptr_t>(base)] = VmmRange{size, mem};
+    }
+    *out = reinterpret_cast<void*>(base);
+    return true;
+}
+
+// Unlike cudaFree, cuMemUnmap does not wait for work still using the range: the device is
+// synchronised first.
+static int vmm_unmap(blf_ccm_handle* h, uintptr_t base, const VmmRange& r)
+{
+    CUDA_TRY(cudaDeviceSynchronize());
+    const VmmApi& api = vmm_api();
+    CUresult e = api.unmap(base, r.size);
+    if (e == CUDA_SUCCESS) e = api.address_free(base, r.size);
+    if (e == CUDA_SUCCESS) e = api.release(r.mem);
+    if (e != CUDA_SUCCESS) return fail(BLF_CCM_ERR_CUDA, "releasing a compressible allocation: CUresult %d", int(e));
+    return BLF_CCM_OK;
+}
+
+static void vmm_release_all(blf_ccm_handle* h)
+{
+    std::lock_guard<std::mutex> lock(h->vmm_mutex);
+    for (const auto& kv : h->vmm) vmm_unmap(h, kv.first, kv.second);
+    h->vmm.clear();
+}
+
+extern "C" int blf_ccm_device_alloc_compressible(blf_ccm_handle* h, uint64_t bytes, void** out, int* granted)
+{
+    CHECK_HANDLE(h);
+    if (!out) return fail(BLF_CCM_ERR_INVALID_ARG, "out is NULL");
+    *out = nullptr;
+    if (granted) *granted = 0;
+    if (bytes == 0) return BLF_CCM_OK;
+    CUDA_TRY(cudaFree(nullptr));   // the driver calls below need the device's primary context current
+    if (vmm_map_compressible(h, bytes, out)) {
+        if (granted) *granted = 1;
+        return BLF_CCM_OK;
+    }
+    CUDA_TRY(cudaMalloc(out, bytes));
+    return BLF_CCM_OK;
+}
+
+extern "C" int blf_ccm_pointer_is_compressible(blf_ccm_handle* h, const void* ptr, int* out)
+{
+    CHECK_HANDLE(h);
+    if (!out) return fail(BLF_CCM_ERR_INVALID_ARG, "out is NULL");
+    const uintptr_t p = reinterpret_cast<uintptr_t>(ptr);
+    std::lock_guard<std::mutex> lock(h->vmm_mutex);
+    auto it = h->vmm.upper_bound(p);
+    *out = it != h->vmm.begin() && p < std::prev(it)->first + std::prev(it)->second.size;
+    return BLF_CCM_OK;
+}
+
 extern "C" int blf_ccm_device_free(blf_ccm_handle* h, void* ptr)
 {
     CHECK_HANDLE(h);
-    if (ptr) CUDA_TRY(cudaFree(ptr));
+    if (!ptr) return BLF_CCM_OK;
+    {
+        std::lock_guard<std::mutex> lock(h->vmm_mutex);
+        auto it = h->vmm.find(reinterpret_cast<uintptr_t>(ptr));
+        if (it != h->vmm.end()) {
+            const VmmRange r = it->second;
+            h->vmm.erase(it);
+            return vmm_unmap(h, reinterpret_cast<uintptr_t>(ptr), r);
+        }
+    }
+    CUDA_TRY(cudaFree(ptr));
     return BLF_CCM_OK;
 }
 

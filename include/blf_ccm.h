@@ -436,7 +436,23 @@ BLF_CCM_API int blf_sys_floating_base_euler_step(blf_ccm_handle* h, int64_t n_sy
  * aligned.  Copies are asynchronous on `stream` when the host side is pinned.
  */
 BLF_CCM_API int blf_ccm_device_alloc(blf_ccm_handle* h, uint64_t bytes, void** out);
+/* Frees memory from blf_ccm_device_alloc or blf_ccm_device_alloc_compressible.  A compressible
+ * allocation is released after a device synchronise (the driver's unmap, unlike cudaFree, does not
+ * wait for kernels still using it). */
 BLF_CCM_API int blf_ccm_device_free(blf_ccm_handle* h, void* ptr);
+/*
+ * Device memory with Compute Data Compression requested (cuMemCreate, CU_MEM_ALLOCATION_COMP_GENERIC),
+ * meant for the dense n x 36 control-matrix array: 24 of its 36 entries are structural +0.0, and the
+ * memory system can keep such data compressed between L2 and HBM.  Compression is invisible to every
+ * reader (kernels, copies): the values are the ones written.  *granted (may be NULL) is 1 when the
+ * driver granted compression; when the device has no compression or the driver does not grant it,
+ * the memory comes from cudaMalloc and *granted is 0.  The size is rounded up to the allocation
+ * granularity; the base is at least 256-byte aligned.  Free with blf_ccm_device_free.
+ */
+BLF_CCM_API int blf_ccm_device_alloc_compressible(blf_ccm_handle* h, uint64_t bytes, void** out,
+                                                  int* granted);
+/* *out = 1 when ptr lies inside a live compressible allocation of this handle, else 0. */
+BLF_CCM_API int blf_ccm_pointer_is_compressible(blf_ccm_handle* h, const void* ptr, int* out);
 BLF_CCM_API int blf_ccm_host_alloc(blf_ccm_handle* h, uint64_t bytes, void** out); /* pinned */
 BLF_CCM_API int blf_ccm_host_free(blf_ccm_handle* h, void* ptr);
 BLF_CCM_API int blf_ccm_copy_h2d(blf_ccm_handle* h, void* dst_device, const void* src_host,
