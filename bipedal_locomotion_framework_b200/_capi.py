@@ -18,7 +18,8 @@ OK, ERR_INVALID_ARG, ERR_INVALID_HANDLE, ERR_CUDA, ERR_NO_DEVICE, ERR_NOT_INITIA
 # every symbol include/blf_ccm.h declares
 SYMBOLS = [
     "blf_ccm_version", "blf_ccm_last_error", "blf_ccm_create", "blf_ccm_destroy",
-    "blf_ccm_set_uniform_params", "blf_ccm_eval_batch_soa", "blf_ccm_eval_batch_aos",
+    "blf_ccm_set_uniform_params", "blf_ccm_eval_batch_soa", "blf_ccm_wrench_vjp_soa",
+    "blf_ccm_eval_batch_aos",
     "blf_ccm_eval_batch_host", "blf_ccm_set_host_chunk", "blf_ccm_set_host_threads",
     "blf_ccm_eval_surface_points",
     "blf_ccm_rollout_cost_argmin_soa", "blf_ccm_argmin_pairs", "blf_ccm_argmin_allgather_nccl",
@@ -61,6 +62,7 @@ def lib():
     L.blf_ccm_destroy.argtypes = [vp]
     L.blf_ccm_set_uniform_params.argtypes = [vp, dbl, dbl, dbl, dbl]
     L.blf_ccm_eval_batch_soa.argtypes = [vp, i64, vp, vp, u32, vp, vp, vp, vp, vp]
+    L.blf_ccm_wrench_vjp_soa.argtypes = [vp, i64, vp, vp, vp, vp, vp, vp]
     L.blf_ccm_eval_batch_aos.argtypes = [vp, i64, vp, vp, vp, vp, u32, vp, vp, vp, vp, vp]
     L.blf_ccm_eval_batch_host.argtypes = [vp, i64, vp, vp, vp, vp, u32, vp, vp, vp, vp]
     L.blf_ccm_set_host_chunk.argtypes = [vp, i64]

@@ -87,6 +87,7 @@ CPP_TESTS = {
     "ContactWrenchUnitTests": "ContactWrenchTest.cpp",                     # host only
     "FloatingBaseSystemDynamicsUnitTests": "FloatingBaseSystemDynamicsTest.cpp",   # needs a GPU
     "ApiConformanceUnitTests": "ApiConformanceTest.cpp",                   # compile-time signature checks
+    "ContactWrenchGradientUnitTests": "ContactWrenchGradientTest.cpp",     # needs a GPU
 }
 CXX_FLAGS = ["-std=c++17", "-O2", "-fPIC", "-Wall", "-Wextra"]
 

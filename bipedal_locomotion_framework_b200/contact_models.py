@@ -321,6 +321,55 @@ class ContinuousContactModel:
 # batched entry point
 # --------------------------------------------------------------------------------------------------
 
+# gradient groups of blf_ccm_wrench_vjp_soa: the state planes each one covers
+VJP_GROUPS = {"twist": slice(0, 6), "pose": slice(6, 18), "null_pose": slice(18, 30)}
+
+_CONTACT_WRENCH_FN = None
+
+
+def _contact_wrench_function():
+    """torch.autograd.Function of ContinuousContactModelBatch.contact_wrench (built on first use, so
+    importing this module does not import torch)."""
+    global _CONTACT_WRENCH_FN
+    if _CONTACT_WRENCH_FN is not None:
+        return _CONTACT_WRENCH_FN
+    import torch
+    from torch.autograd.function import once_differentiable
+
+    class ContactWrench(torch.autograd.Function):
+        @staticmethod
+        def forward(ctx, batch, param_planes, *planes):
+            state = planes if len(planes) == 30 else planes[0]
+            ctx.batch = batch
+            ctx.save_for_backward(param_planes, *planes)
+            return batch.evaluate_soa(state, param_planes, WRENCH,
+                                      out=batch.alloc_soa_outputs(batch._num_contacts(state), WRENCH))["wrench"]
+
+        @staticmethod
+        @once_differentiable
+        def backward(ctx, grad_wrench):
+            batch = ctx.batch
+            param_planes, *planes = ctx.saved_tensors
+            state = planes if len(planes) == 30 else planes[0]
+            need_state = ctx.needs_input_grad[2:]
+            if len(planes) == 30:
+                groups = {g for g, rows in VJP_GROUPS.items() if any(need_state[rows])}
+            else:
+                groups = set(VJP_GROUPS) if need_state[0] else set()
+            want_params = ctx.needs_input_grad[1]
+            if not groups and not want_params:
+                return (None,) * (2 + len(planes))
+            g = batch.wrench_vjp(state, grad_wrench.contiguous(), param_planes, inputs=groups,
+                                 params=want_params)
+            if len(planes) == 30:
+                gs = [g["planes"][i] if need_state[i] else None for i in range(30)]
+            else:
+                gs = [g["planes"] if need_state[0] else None]
+            return (None, g["params"]) + tuple(gs)
+
+    _CONTACT_WRENCH_FN = ContactWrench
+    return ContactWrench
+
 class ContinuousContactModelBatch:
     """Batched evaluation on one GPU.  Inputs/outputs are torch CUDA tensors (float64) or, for
     evaluate_host, numpy arrays; all arithmetic happens in libblf_ccm.so."""
@@ -442,6 +491,65 @@ class ContinuousContactModelBatch:
             if rc:
                 _capi.check(rc)
         return call, out
+
+    def _vjp_args(self, planes, grad_wrench, param_planes, inputs, params, out):
+        """Arguments of blf_ccm_wrench_vjp_soa and the output dict (see wrench_vjp)."""
+        t = self._torch
+        n = self._num_contacts(planes)
+        groups = set(VJP_GROUPS) if inputs is True else set(inputs or ())
+        assert groups <= set(VJP_GROUPS), f"unknown gradient groups {groups - set(VJP_GROUPS)}"
+        if out is None:
+            out = {"planes": t.empty((30, n), dtype=t.float64, device=self.device) if groups else None,
+                   "params": t.empty((4, n), dtype=t.float64, device=self.device) if params else None}
+        gin = None
+        if groups:
+            # planes of groups that were not asked for are neither computed nor written: zero them
+            for name, rows in VJP_GROUPS.items():
+                if name not in groups:
+                    out["planes"][rows].zero_()
+            live = {i for g in groups for i in range(30)[VJP_GROUPS[g]]}
+            gin = _ptr_array([out["planes"][i].data_ptr() if i in live else None for i in range(30)])
+        args = (self._handle.ptr, n, self._plane_ptrs(planes, 30), self._plane_ptrs(param_planes, 4),
+                self._plane_ptrs(grad_wrench, 6), gin, self._plane_ptrs(out["params"], 4),
+                self._stream())
+        return args, out
+
+    def wrench_vjp(self, planes, grad_wrench, param_planes=None, inputs=True, params: bool = False,
+                   out: dict | None = None) -> dict:
+        """Reverse mode of the contact wrench (blf_ccm_wrench_vjp_soa): for the (6, n) cotangent
+        `grad_wrench` (rows force xyz, torque xyz) returns {"planes": (30, n) gbar^T dwrench/dstate or
+        None, "params": (4, n) per-contact gbar^T dwrench/d(length, width, spring, damper) or None}.
+        `inputs`: True for every state plane, False for none, or a subset of "twist", "pose",
+        "null_pose"; the planes of other groups are returned as zeros.  With uniform parameters
+        the sum over contacts of "params" is the gradient of the shared values."""
+        args, out = self._vjp_args(planes, grad_wrench, param_planes, inputs, params, out)
+        _capi.check(_capi.lib().blf_ccm_wrench_vjp_soa(*args))
+        return out
+
+    def prepare_wrench_vjp(self, planes, grad_wrench, param_planes=None, inputs=True,
+                           params: bool = False, out: dict | None = None):
+        """Prepared form of wrench_vjp (every argument bound once).  Returns (call, out)."""
+        args, out = self._vjp_args(planes, grad_wrench, param_planes, inputs, params, out)
+        fn = _capi.lib().blf_ccm_wrench_vjp_soa
+        keep = (planes, grad_wrench, param_planes, out)
+
+        def call(_keep=keep):
+            rc = fn(*args)
+            if rc:
+                _capi.check(rc)
+        return call, out
+
+    def contact_wrench(self, planes, param_planes=None):
+        """(6, n) contact wrench (rows force xyz, torque xyz) of the (30, n) state planes, through
+        torch.autograd: gradients reach `planes` and `param_planes` (4, n) when they require them.
+        `planes` may also be a list of 30 1-D tensors (dead planes None); then only the gradient
+        groups (twist, pose, null pose) of planes that require grad are computed.  The backward is
+        blf_ccm_wrench_vjp_soa; it is not itself differentiable."""
+        fn = _contact_wrench_function()
+        if isinstance(planes, (list, tuple)):
+            assert len(planes) == 30
+            return fn.apply(self, param_planes, *planes)
+        return fn.apply(self, param_planes, planes)
 
     def prepare_aos(self, twists, poses, null_poses, params=None, mask: int = FULL,
                     out: dict | None = None):

@@ -121,6 +121,23 @@ public:
                   GenericContainer::DeviceSoA* regressor, void* stream = nullptr);
 
     /**
+     * Reverse mode of the contact wrench (asynchronous on `stream`): for per-contact cotangents
+     * of the wrench, the vector-Jacobian products with respect to the state and the parameters.
+     * @param states 30 planes (Plane order); planes no requested gradient reads may be null
+     * @param parameters 4 planes length,width,spring,damper or nullptr for the uniform ones
+     * @param wrenchCotangent 6 planes force xyz, torque xyz; a null plane counts as zero
+     * @param stateGradient 30 planes or nullptr; every non-null plane is written (R02, R12 and the
+     *        null-force rotation's third column with +0.0), the others are neither computed nor written
+     * @param parameterGradient 4 planes or nullptr: each contact's gradient with respect to
+     *        length, width, spring, damper (with uniform parameters, their sum over contacts)
+     */
+    bool wrenchGradient(const GenericContainer::DeviceSoA& states,
+                        const GenericContainer::DeviceSoA* parameters,
+                        const GenericContainer::DeviceSoA& wrenchCotangent,
+                        GenericContainer::DeviceSoA* stateGradient,
+                        GenericContainer::DeviceSoA* parameterGradient, void* stream = nullptr);
+
+    /**
      * Host arrays of iDynTree objects in, host arrays of iDynTree objects out (what a loop over
      * ContactModel instances would produce).  Copies and kernels are pipelined; returns when the
      * results are in host memory.

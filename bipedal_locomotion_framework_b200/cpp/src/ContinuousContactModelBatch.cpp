@@ -146,6 +146,36 @@ bool ContinuousContactModelBatch::evaluate(const DeviceSoA& states, const Device
                   "evaluate");
 }
 
+bool ContinuousContactModelBatch::wrenchGradient(const DeviceSoA& states, const DeviceSoA* parameters,
+                                                 const DeviceSoA& wrenchCotangent,
+                                                 DeviceSoA* stateGradient, DeviceSoA* parameterGradient,
+                                                 void* stream)
+{
+    if (m_device == nullptr) return report(BLF_CCM_ERR_INVALID_HANDLE, "wrenchGradient");
+    const bool shapes = states.planes() == NumberOfPlanes && wrenchCotangent.planes() == 6
+                        && wrenchCotangent.size() == states.size()
+                        && (parameters == nullptr || (parameters->planes() == 4 && parameters->size() == states.size()))
+                        && (stateGradient == nullptr
+                            || (stateGradient->planes() == NumberOfPlanes && stateGradient->size() == states.size()))
+                        && (parameterGradient == nullptr
+                            || (parameterGradient->planes() == 4 && parameterGradient->size() == states.size()));
+    if (!shapes)
+    {
+        std::cerr << "[ContinuousContactModelBatch::wrenchGradient] states and stateGradient must have 30 "
+                     "planes, wrenchCotangent 6, parameters and parameterGradient 4, all of the same size."
+                  << std::endl;
+        return false;
+    }
+    return report(blf_ccm_wrench_vjp_soa(raw(m_device), static_cast<std::int64_t>(states.size()),
+                                         states.planePointers(),
+                                         parameters ? parameters->planePointers() : nullptr,
+                                         wrenchCotangent.planePointers(),
+                                         stateGradient ? stateGradient->planePointers() : nullptr,
+                                         parameterGradient ? parameterGradient->planePointers() : nullptr,
+                                         stream),
+                  "wrenchGradient");
+}
+
 bool ContinuousContactModelBatch::evaluate(std::size_t n, const iDynTree::Twist* twists,
                                            const iDynTree::Transform* transforms,
                                            const iDynTree::Transform* nullForceTransforms,

@@ -532,6 +532,82 @@ extern "C" int blf_ccm_eval_batch_soa(blf_ccm_handle* h, int64_t n, const double
     return dispatch_mask<SoaLaunch, false>(out_mask, h, a, vec2, st);
 }
 
+// ---- reverse mode of the wrench --------------------------------------------------------------------
+
+template <unsigned GROUPS, bool HET>
+struct VjpLaunch {
+    static int run(blf_ccm_handle* h, const VjpArgs& a, cudaStream_t st)
+    {
+        constexpr int threads = 128;
+        const long long grid = (a.n + threads - 1) / threads;
+        if (grid > 0x7fffffffLL) return fail(BLF_CCM_ERR_INVALID_ARG, "n too large for one launch");
+        CUDA_TRY(launch_pdl(h, ccm_wrench_vjp_kernel<GROUPS, HET>, grid, threads, 0, st, a));
+        CUDA_TRY(cudaGetLastError());
+        h->launches++;
+        return BLF_CCM_OK;
+    }
+};
+
+extern "C" int blf_ccm_wrench_vjp_soa(blf_ccm_handle* h, int64_t n, const double* const* in_planes,
+                                      const double* const* param_planes,
+                                      const double* const* grad_wrench_planes,
+                                      double* const* grad_in_planes, double* const* grad_param_planes,
+                                      void* stream)
+{
+    CHECK_HANDLE(h);
+    if (n < 0) return fail(BLF_CCM_ERR_INVALID_ARG, "n < 0");
+    unsigned groups = grad_param_planes ? G_PARAMS : 0u;
+    if (grad_in_planes)
+        for (int i = 0; i < 30; ++i)
+            if (grad_in_planes[i])
+                for (unsigned g : {G_TWIST, G_POSE, G_NULL})
+                    if (vjp_group_planes(g) & (1u << i)) groups |= g;
+    if (groups == 0) return fail(BLF_CCM_ERR_INVALID_ARG, "no gradient requested");
+    if (n == 0) return BLF_CCM_OK;  // empty batch: nothing to read, nothing to write
+    if (!in_planes) return fail(BLF_CCM_ERR_INVALID_ARG, "in_planes is NULL");
+    if (!param_planes && !h->have_params)
+        return fail(BLF_CCM_ERR_NOT_INITIALIZED,
+                    "no parameters: call blf_ccm_set_uniform_params or pass param_planes");
+    VjpArgs a;
+    memset(&a, 0, sizeof(a));
+    a.n = n;
+    a.uni[0] = h->length;
+    a.uni[1] = h->width;
+    a.uni[2] = h->spring;
+    a.uni[3] = h->damper;
+    const unsigned live = vjp_live_planes(groups);
+    for (int i = 0; i < 30; ++i) {
+        if (!(live & (1u << i))) continue;
+        if (!in_planes[i])
+            return fail(BLF_CCM_ERR_INVALID_ARG, "in_planes[%d] is NULL but read for the requested gradients", i);
+        if (!aligned8(in_planes[i])) return fail(BLF_CCM_ERR_INVALID_ARG, "in_planes[%d] not 8-byte aligned", i);
+        a.in[i] = in_planes[i];
+    }
+    auto take = [&](const double* const* src, const double** dst, int cnt, bool nullable,
+                    const char* what) -> int {
+        for (int i = 0; i < cnt; ++i) {
+            if (!src[i] && nullable) continue;
+            if (!src[i] || !aligned8(src[i]))
+                return fail(BLF_CCM_ERR_INVALID_ARG, "%s[%d] NULL or misaligned", what, i);
+            dst[i] = src[i];
+        }
+        return BLF_CCM_OK;
+    };
+    if (param_planes)
+        if (int rc = take(param_planes, a.prm, 4, false, "param_planes")) return rc;
+    if (grad_wrench_planes)
+        if (int rc = take(grad_wrench_planes, a.gw, 6, true, "grad_wrench_planes")) return rc;
+    if (grad_in_planes)
+        if (int rc = take(grad_in_planes, const_cast<const double**>(a.gin), 30, true, "grad_in_planes"))
+            return rc;
+    if (grad_param_planes)
+        if (int rc = take(grad_param_planes, const_cast<const double**>(a.gprm), 4, false, "grad_param_planes"))
+            return rc;
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    if (param_planes) return dispatch_mask<VjpLaunch, true>(groups, h, a, st);
+    return dispatch_mask<VjpLaunch, false>(groups, h, a, st);
+}
+
 // ---- AoS -----------------------------------------------------------------------------------------
 
 template <unsigned MASK, bool HET>

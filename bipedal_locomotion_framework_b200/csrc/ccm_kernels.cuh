@@ -765,6 +765,95 @@ __device__ __forceinline__ CostIdx warp_best(CostIdx b)
     return b;
 }
 
+// ------------------------------------------------------------------------------------------------
+// Reverse mode of the wrench (vector-Jacobian product), organised as ccm_soa_kernel: one contact
+// per lane, one 32-contact tile per warp, every live plane in flight before the first use,
+// streaming 64-bit loads and stores.  GROUPS (G_TWIST | G_POSE | G_NULL | G_PARAMS) selects the
+// gradients computed; only the input planes those need are read.
+// ------------------------------------------------------------------------------------------------
+
+struct VjpArgs {
+    const double* in[30];
+    const double* prm[4];      // length, width, spring, damper planes (HET only)
+    const double* gw[6];       // cotangent planes gF, gT; nullptr = zero
+    double* gin[30];           // gradient planes of the state; nullptr = not written
+    double* gprm[4];           // per-contact gradient of length, width, spring, damper (G_PARAMS)
+    double uni[4];             // uniform length, width, spring, damper
+    long long n;
+};
+
+template <unsigned GROUPS, bool HET>
+__global__ void __launch_bounds__(128)
+ccm_wrench_vjp_kernel(const __grid_constant__ VjpArgs a)
+{
+    constexpr unsigned LIVE = vjp_live_planes(GROUPS);
+    const int lane = threadIdx.x & 31;
+    const long long tile = static_cast<long long>(blockIdx.x) * (blockDim.x >> 5) + (threadIdx.x >> 5);
+    const long long base = tile << 5;
+    if (base >= a.n) return;  // warp-uniform
+    const long long i = base + lane;
+    const bool on = i < a.n;
+
+    ptx::grid_dep_launch_dependents();
+    ptx::grid_dep_wait();
+
+    double x[30] = {};
+#pragma unroll
+    for (int pl = 0; pl < 30; ++pl)
+        if (LIVE & (1u << pl)) x[pl] = on ? __ldcs(a.in[pl] + i) : 0.0;
+    double gw[6];
+#pragma unroll
+    for (int j = 0; j < 6; ++j) gw[j] = (on && a.gw[j]) ? __ldcs(a.gw[j] + i) : 0.0;
+    double l = a.uni[0], w = a.uni[1], k = a.uni[2], b = a.uni[3];
+    if constexpr (HET) {
+        l = on ? __ldcs(a.prm[0] + i) : 0.0;
+        w = on ? __ldcs(a.prm[1] + i) : 0.0;
+        k = on ? __ldcs(a.prm[2] + i) : 0.0;
+        b = on ? __ldcs(a.prm[3] + i) : 0.0;
+    }
+    const Prm q = make_prm(l, w, k, b);
+
+    State s;
+    s.v = V3{x[0], x[1], x[2]};
+    s.w = V3{x[3], x[4], x[5]};
+    s.p = V3{x[6], x[7], x[8]};
+    s.e1 = V3{x[9], x[12], x[15]};
+    s.e2 = V3{x[10], x[13], x[16]};
+    s.R02 = 0.0;
+    s.R12 = 0.0;
+    s.R22 = x[17];
+    s.p0 = V3{x[18], x[19], x[20]};
+    s.n1 = V3{x[21], x[24], x[27]};
+    s.n2 = V3{x[22], x[25], x[28]};
+    VjpOut g;
+    vjp_wrench<GROUPS>(s, q, l, w, V3{gw[0], gw[1], gw[2]}, V3{gw[3], gw[4], gw[5]}, g);
+    if (!on) return;
+
+    auto put = [&](int pl, double val) {
+        if (a.gin[pl]) __stcs(a.gin[pl] + i, val);
+    };
+    if constexpr ((GROUPS & G_TWIST) != 0) {
+        put(0, g.v.x); put(1, g.v.y); put(2, g.v.z);
+        put(3, g.w.x); put(4, g.w.y); put(5, g.w.z);
+    }
+    if constexpr ((GROUPS & G_POSE) != 0) {
+        put(6, g.p.x); put(7, g.p.y); put(8, g.p.z);
+        put(9, g.e1.x); put(10, g.e2.x); put(11, 0.0);
+        put(12, g.e1.y); put(13, g.e2.y); put(14, 0.0);
+        put(15, g.e1.z); put(16, g.e2.z); put(17, g.R22);
+    }
+    if constexpr ((GROUPS & G_NULL) != 0) {
+        put(18, g.p0.x); put(19, g.p0.y); put(20, g.p0.z);
+        put(21, g.n1.x); put(22, g.n2.x); put(23, 0.0);
+        put(24, g.n1.y); put(25, g.n2.y); put(26, 0.0);
+        put(27, g.n1.z); put(28, g.n2.z); put(29, 0.0);
+    }
+    if constexpr ((GROUPS & G_PARAMS) != 0) {
+        __stcs(a.gprm[0] + i, g.L); __stcs(a.gprm[1] + i, g.W);
+        __stcs(a.gprm[2] + i, g.k); __stcs(a.gprm[3] + i, g.b);
+    }
+}
+
 }  // namespace blfccm
 #include "p2p_kernels.cuh"
 namespace blfccm {

@@ -172,4 +172,102 @@ __host__ __device__ constexpr unsigned live_planes(unsigned mask)
     return all;
 }
 
+// ------------------------------------------------------------------------------------------------
+// Reverse mode of the wrench: gbar^T d(wrench)/d(inputs) for a cotangent gbar = (gF, gT).
+// With ac = |R22|, alpha = ac A, beta = ac A/12, sd = k (p0 - p) - b v, u_i = e_i x (e_i x w),
+// m_i = e_i x n_i, T_i = b u_i + k m_i, Tb = L^2 T1 + W^2 T2 and h1 = beta L^2 gT, h2 = beta W^2 gT:
+//   p0: k alpha gF        p: -k alpha gF        v: -b alpha gF
+//   w:  b sum_i e_i x (e_i x h_i)                         (S(e)^2 is symmetric)
+//   e_i: b [h_i (e_i.w) + w (h_i.e_i) - 2 (h_i.w) e_i] + k n_i x h_i
+//   n_i: k h_i x e_i
+//   R22: sgn(R22) (A gF.sd + A/12 gT.Tb), sgn(+-0) = 0 (torch.abs's backward)
+//   k: gF.y_fk + gT.y_tk    b: gF.y_fb + gT.y_tb          (the regressor columns)
+//   L: ac W gF.sd + ac W/12 gT.Tb + 2 L beta gT.T1        W: same with L <-> W, T2.
+// R02, R12 and R0's third column do not enter the wrench: their gradient is structurally zero.
+// ------------------------------------------------------------------------------------------------
+
+// gradient groups (bits of the GROUPS template argument and of vjp_live_planes)
+enum : unsigned { G_TWIST = 1u, G_POSE = 2u, G_NULL = 4u, G_PARAMS = 8u };
+
+struct VjpOut {
+    V3 v, w, p, e1, e2, p0, n1, n2;
+    double R22;
+    double L, W, k, b;   // length, width, spring, damper
+};
+
+__device__ __forceinline__ double dot(const V3& a, const V3& b) { return a.x * b.x + a.y * b.y + a.z * b.z; }
+
+template <unsigned G>
+__device__ __forceinline__ void vjp_wrench(const State& s, const Prm& q, double length, double width,
+                                           const V3& gF, const V3& gT, VjpOut& g)
+{
+    constexpr bool kTw = (G & G_TWIST) != 0;
+    constexpr bool kPo = (G & G_POSE) != 0;
+    constexpr bool kNu = (G & G_NULL) != 0;
+    constexpr bool kPa = (G & G_PARAMS) != 0;
+
+    const double c = s.R22;
+    const double ac = fabs(c);
+    const double alpha = ac * q.A, beta = ac * q.A12;
+    const V3 h1 = (beta * q.L2) * gT, h2 = (beta * q.W2) * gT;
+
+    if constexpr (kTw) {
+        g.v = (-(q.b * alpha)) * gF;
+        g.w = q.b * (cross(s.e1, cross(s.e1, h1)) + cross(s.e2, cross(s.e2, h2)));
+    }
+    if constexpr (kPo || kNu) {
+        const V3 gp0 = (q.k * alpha) * gF;
+        if constexpr (kNu) {
+            g.p0 = gp0;
+            g.n1 = q.k * cross(h1, s.e1);
+            g.n2 = q.k * cross(h2, s.e2);
+        }
+        if constexpr (kPo) g.p = neg(gp0);
+    }
+    if constexpr (kPo) {
+        const double ew1 = dot(s.e1, s.w), hw1 = dot(h1, s.w), he1 = dot(h1, s.e1);
+        const double ew2 = dot(s.e2, s.w), hw2 = dot(h2, s.w), he2 = dot(h2, s.e2);
+        g.e1 = q.b * (ew1 * h1 + he1 * s.w - (2.0 * hw1) * s.e1) + q.k * cross(s.n1, h1);
+        g.e2 = q.b * (ew2 * h2 + he2 * s.w - (2.0 * hw2) * s.e2) + q.k * cross(s.n2, h2);
+    }
+    if constexpr (kPo || kPa) {
+        const V3 d = s.p0 - s.p;
+        const V3 sd = q.k * d - q.b * s.v;
+        const V3 u1 = cross(s.e1, cross(s.e1, s.w)), u2 = cross(s.e2, cross(s.e2, s.w));
+        const V3 m1 = cross_exact(s.e1, s.n1), m2 = cross_exact(s.e2, s.n2);
+        const double fs = dot(gF, sd);
+        const double t1 = dot(gT, q.b * u1 + q.k * m1), t2 = dot(gT, q.b * u2 + q.k * m2);
+        const double ts = q.L2 * t1 + q.W2 * t2;   // gT.Tb
+        if constexpr (kPo) {
+            const double sg = c > 0.0 ? 1.0 : (c < 0.0 ? -1.0 : 0.0);
+            g.R22 = sg * (q.A * fs + q.A12 * ts);
+        }
+        if constexpr (kPa) {
+            g.k = alpha * dot(gF, d) + beta * (q.L2 * dot(gT, m1) + q.W2 * dot(gT, m2));
+            g.b = -alpha * dot(gF, s.v) + beta * (q.L2 * dot(gT, u1) + q.W2 * dot(gT, u2));
+            g.L = ac * width * (fs + ts / 12.0) + (2.0 * length * beta) * t1;
+            g.W = ac * length * (fs + ts / 12.0) + (2.0 * width * beta) * t2;
+        }
+    }
+}
+
+// Which of the 30 SoA input planes the requested gradient groups read (bit i = plane i).  The
+// cotangents (and, with per-contact parameters, the 4 parameter planes) are read by every group.
+__host__ __device__ constexpr unsigned vjp_live_planes(unsigned groups)
+{
+    const unsigned all = live_planes(M_WRENCH);   // the 25 planes the wrench depends on
+    const unsigned e12 = (1u << 9) | (1u << 10) | (1u << 12) | (1u << 13) | (1u << 15) | (1u << 16);
+    const unsigned r22 = 1u << 17;
+    unsigned live = 0;
+    if (groups & (G_POSE | G_PARAMS)) live |= all;
+    if (groups & (G_TWIST | G_NULL)) live |= e12 | r22;
+    return live;
+}
+
+// The input planes of each gradient group: twist 0-5, pose 6-17, null pose 18-29.
+__host__ __device__ constexpr unsigned vjp_group_planes(unsigned group)
+{
+    return group == G_TWIST ? 0x3Fu : group == G_POSE ? 0x3FFC0u : group == G_NULL ? 0x3FFC0000u : 0u;
+}
+
 }  // namespace blfccm

@@ -129,6 +129,27 @@ BLF_CCM_API int blf_ccm_eval_batch_soa(blf_ccm_handle* h, int64_t n,
                                        double* const* autodyn_planes, double* ctrl,
                                        double* const* regressor_planes, void* stream);
 
+/* Reverse mode of the contact wrench (ContinuousContactModel.cpp:79-108; no reference
+ * counterpart computes it): for per-contact cotangents gbar = (gF, gT) of the wrench, writes
+ * gbar^T d(wrench)/d(state) and gbar^T d(wrench)/d(length, width, spring, damper).
+ *   in_planes           30 planes as blf_ccm_eval_batch_soa; planes no requested gradient reads may
+ *                       be NULL (twist and null-pose gradients read only R's first two columns and R22)
+ *   param_planes        4 planes length,width,spring,damper, or NULL for the uniform parameters
+ *   grad_wrench_planes  6 cotangent planes force xyz, torque xyz; NULL (or a NULL entry) counts as zero
+ *   grad_in_planes      30 planes or NULL; every non-NULL entry is written, and it requests the
+ *                       gradient of its group: twist (0-5), pose (6-17), null pose (18-29).  R02, R12
+ *                       and R0's third column (11, 14, 23, 26, 29) do not enter the wrench: +0.0.
+ *   grad_param_planes   4 planes or NULL: each contact's contribution to the gradient of its
+ *                       parameters; with uniform parameters their sum is the shared value's gradient.
+ * The derivative of |R22| at R22 = +-0 is taken as 0.  Nothing requested, n < 0, or a NULL plane that
+ * a requested gradient reads is BLF_CCM_ERR_INVALID_ARG; n = 0 is a no-op.  One launch. */
+BLF_CCM_API int blf_ccm_wrench_vjp_soa(blf_ccm_handle* h, int64_t n,
+                                       const double* const* in_planes,
+                                       const double* const* param_planes,
+                                       const double* const* grad_wrench_planes,
+                                       double* const* grad_in_planes,
+                                       double* const* grad_param_planes, void* stream);
+
 /* Array-of-structures evaluation: arrays of iDynTree-layout objects in, arrays of
  * iDynTree-layout objects out.  twists n*6, poses n*12, null_poses n*12, params NULL or n structs;
  * wrench n*6, autodyn n*6, ctrl n*36, regressor n*12 (NULL when not in out_mask). */
