@@ -16,6 +16,7 @@
 #include <map>
 #include <mutex>
 #include <new>
+#include <set>
 #include <type_traits>
 
 #include "ccm_kernels.cuh"
@@ -60,10 +61,6 @@ static constexpr int kHostUpStreamsAuto = 1;
 static constexpr int kStageSlots = 8;    // pinned staging chunks of the compact control-matrix download
 static constexpr int kMaxPartials = 8192;
 
-struct KernelInfo {
-    int blocks_per_sm = 0;
-};
-
 struct TensorMapEntry {
     const double* ptr = nullptr;
     int horizon = 0;
@@ -88,7 +85,7 @@ struct blf_ccm_handle {
     Prm uni{};
     int last_path = BLF_CCM_PATH_NONE;
     long long launches = 0;
-    std::map<const void*, KernelInfo> kinfo;
+    std::set<const void*> prepared;   // kernels prepare_kernel has checked
     // rollout scratch (block_best, counter, partials): ONE set per handle.  Calls that use it on
     // different streams are ordered by the library (scratch_acquire), they never overlap.
     CostIdx* block_best = nullptr;   // kMaxPartials pairs
@@ -120,9 +117,6 @@ struct blf_ccm_handle {
     size_t hbytes = 0;
     long long host_chunk_pref = 131072;   // measured: profiles/r02_host_sweep.log
     // tuning overrides (environment, read once at create; 0 = automatic)
-    int tune_cpt = 0;            // BLF_CCM_TUNE_CPT=2: use the 128-bit two-contacts-per-lane SoA kernel
-    int tune_blocks_per_sm = 0;  // BLF_CCM_TUNE_BLOCKS_PER_SM>0: persistent grid with that many CTAs/SM
-                                 // (looping kernels only); default = one tile per warp
     int tune_rollout_split = 0;  // BLF_CCM_TUNE_ROLLOUT_SPLIT>0: warps per tile of the fused rollout
     int tune_rollout_ws = 0;     // BLF_CCM_TUNE_ROLLOUT_WS: 1 force / 2 forbid the warp-specialised rollout
     int tune_no_pack = 0;        // BLF_CCM_TUNE_NO_PACK=1: J^T wrench for narrow Jacobians with the column-per-lane kernel
@@ -238,10 +232,8 @@ extern "C" int blf_ccm_create(int device, blf_ccm_handle** out)
     h->device = device;
     h->sm_count = prop.multiProcessorCount;
     h->mem_pitch = prop.memPitch;
-    h->tune_cpt = env_int("BLF_CCM_TUNE_CPT");
     h->tune_fbd_tile_kb = env_int("BLF_CCM_TUNE_FBD_TILE_KB");
     h->tune_fbd_no_bulk = env_int("BLF_CCM_TUNE_FBD_NO_BULK");
-    h->tune_blocks_per_sm = env_int("BLF_CCM_TUNE_BLOCKS_PER_SM");
     h->tune_rollout_split = env_int("BLF_CCM_TUNE_ROLLOUT_SPLIT");
     h->tune_no_pdl = env_int("BLF_CCM_TUNE_NO_PDL");
     h->tune_host_noexpand = env_int("BLF_CCM_TUNE_HOST_NOEXPAND");
@@ -363,26 +355,21 @@ extern "C" int blf_ccm_sm_count(const blf_ccm_handle* h) { return valid(h) ? h->
 // launch helpers
 // ------------------------------------------------------------------------------------------------
 
+// First use of a kernel on this handle: allow it `smem` bytes of dynamic shared memory and fail if
+// one block of `threads` threads with that much does not fit on an SM.
 template <typename K>
-static int persistent_blocks(blf_ccm_handle* h, K kernel, int threads, size_t smem, int* out)
+static int prepare_kernel(blf_ccm_handle* h, K kernel, int threads, size_t smem)
 {
     const void* key = reinterpret_cast<const void*>(kernel);
-    auto it = h->kinfo.find(key);
-    if (it == h->kinfo.end()) {
-        if (smem > 48 * 1024)
-            CUDA_TRY(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                          static_cast<int>(smem)));
-        KernelInfo ki;
-        CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ki.blocks_per_sm, kernel, threads,
-                                                               smem));
-        if (ki.blocks_per_sm < 1)
-            return fail(BLF_CCM_ERR_CUDA, "kernel does not fit on an SM (threads %d, smem %zu)",
-                        threads, smem);
-        it = h->kinfo.emplace(key, ki).first;
-    }
-    int per_sm = it->second.blocks_per_sm;
-    if (h->tune_blocks_per_sm > 0) per_sm = std::min(per_sm, h->tune_blocks_per_sm);
-    *out = h->tune_blocks_per_sm > 0 ? per_sm * h->sm_count : 0x7fffffff;
+    if (h->prepared.count(key)) return BLF_CCM_OK;
+    if (smem > 48 * 1024)
+        CUDA_TRY(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                      static_cast<int>(smem)));
+    int blocks_per_sm = 0;
+    CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&blocks_per_sm, kernel, threads, smem));
+    if (blocks_per_sm < 1)
+        return fail(BLF_CCM_ERR_CUDA, "kernel does not fit on an SM (threads %d, smem %zu)", threads, smem);
+    h->prepared.insert(key);
     return BLF_CCM_OK;
 }
 
@@ -408,6 +395,21 @@ static cudaError_t launch_pdl(const blf_ccm_handle* h, K kernel, long long grid,
 static bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
 static bool aligned8(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 7u) == 0; }
 
+// Copies `count` plane pointers into a kernel's arguments.  Entries whose bit in `live` is clear are
+// skipped, and so are NULL entries when `nullable`; every other entry must be non-NULL and 8-byte
+// aligned (the kernels read and write planes with 64-bit accesses).
+template <typename S, typename D>
+static int take_planes(const S* src, D* dst, int count, const char* what, unsigned live = ~0u,
+                       bool nullable = false)
+{
+    for (int i = 0; i < count; ++i) {
+        if ((i < 32 && !(live & (1u << i))) || (nullable && !src[i])) continue;
+        if (!src[i] || !aligned8(src[i])) return fail(BLF_CCM_ERR_INVALID_ARG, "%s[%d] NULL or misaligned", what, i);
+        dst[i] = src[i];
+    }
+    return BLF_CCM_OK;
+}
+
 // compile-time dispatch over the 15 non-empty output masks
 template <template <unsigned, bool> class F, bool HET, typename... Args>
 static int dispatch_mask(unsigned mask, Args&&... args)
@@ -429,28 +431,15 @@ static int dispatch_mask(unsigned mask, Args&&... args)
 
 template <unsigned MASK, bool HET>
 struct SoaLaunch {
-    static int run(blf_ccm_handle* h, const SoaArgs& a, bool vec2, cudaStream_t st)
+    static int run(blf_ccm_handle* h, const SoaArgs& a, cudaStream_t st)
     {
         constexpr int threads = 128;
-        if (vec2) {
-            constexpr int TILE = 64;
-            const size_t smem = (MASK & M_CTRL) ? size_t(threads / 32) * TILE * 288 : 0;
-            auto k = ccm_soa_vec2_kernel<MASK, HET>;
-            int cap = 0;
-            if (int rc = persistent_blocks(h, k, threads, smem, &cap)) return rc;
-            const long long tiles = (a.n + TILE - 1) / TILE;
-            const long long want = (tiles + threads / 32 - 1) / (threads / 32);
-            const int grid = static_cast<int>(std::min<long long>(want, cap));
-            k<<<grid, threads, smem, st>>>(a);
-        } else {
-            const size_t smem = (MASK & M_CTRL) ? size_t(threads / 32) * 32 * 288 : 0;
-            auto k = ccm_soa_kernel<MASK, HET, false>;
-            int cap = 0;
-            if (int rc = persistent_blocks(h, k, threads, smem, &cap)) return rc;  // smem attribute
-            const long long grid = (a.n + threads - 1) / threads;
-            if (grid > 0x7fffffffLL) return fail(BLF_CCM_ERR_INVALID_ARG, "n too large for one launch");
-            CUDA_TRY(launch_pdl(h, k, grid, threads, smem, st, a));
-        }
+        const size_t smem = (MASK & M_CTRL) ? size_t(threads / 32) * 32 * 288 : 0;
+        auto k = ccm_soa_kernel<MASK, HET, false>;
+        if (int rc = prepare_kernel(h, k, threads, smem)) return rc;
+        const long long grid = (a.n + threads - 1) / threads;
+        if (grid > 0x7fffffffLL) return fail(BLF_CCM_ERR_INVALID_ARG, "n too large for one launch");
+        CUDA_TRY(launch_pdl(h, k, grid, threads, smem, st, a));
         CUDA_TRY(cudaGetLastError());
         h->launches++;
         return BLF_CCM_OK;
@@ -460,7 +449,7 @@ struct SoaLaunch {
 static int fill_soa_args(blf_ccm_handle* h, long long n, const double* const* in_planes,
                          const double* const* param_planes, unsigned out_mask, unsigned compute_mask,
                          double* const* wrench_planes, double* const* autodyn_planes, double* ctrl,
-                         double* const* regressor_planes, SoaArgs& a, bool& vec)
+                         double* const* regressor_planes, SoaArgs& a)
 {
     if (n < 0) return fail(BLF_CCM_ERR_INVALID_ARG, "n < 0");
     if (!in_planes) return fail(BLF_CCM_ERR_INVALID_ARG, "in_planes is NULL");
@@ -470,43 +459,22 @@ static int fill_soa_args(blf_ccm_handle* h, long long n, const double* const* in
     memset(&a, 0, sizeof(a));
     a.n = n;
     a.uni = h->uni;
-    vec = true;
-    const unsigned live = live_planes(compute_mask);
-    for (int i = 0; i < 30; ++i) {
-        if (!(live & (1u << i))) continue;
-        if (!in_planes[i]) return fail(BLF_CCM_ERR_INVALID_ARG, "in_planes[%d] is NULL but live for out_mask %u", i, out_mask);
-        if (!aligned8(in_planes[i])) return fail(BLF_CCM_ERR_INVALID_ARG, "in_planes[%d] not 8-byte aligned", i);
-        a.in[i] = in_planes[i];
-        vec = vec && aligned16(in_planes[i]);
-    }
+    if (int rc = take_planes(in_planes, a.in, 30, "in_planes", live_planes(compute_mask))) return rc;
     if (param_planes)
-        for (int i = 0; i < 4; ++i) {
-            if (!param_planes[i] || !aligned8(param_planes[i]))
-                return fail(BLF_CCM_ERR_INVALID_ARG, "param_planes[%d] NULL or misaligned", i);
-            a.prm[i] = param_planes[i];
-            vec = vec && aligned16(param_planes[i]);
-        }
-    auto take = [&](double* const* src, double** dst, int cnt, const char* what) -> int {
+        if (int rc = take_planes(param_planes, a.prm, 4, "param_planes")) return rc;
+    auto take_out = [&](double* const* src, double** dst, int cnt, const char* what) -> int {
         if (!src) return fail(BLF_CCM_ERR_INVALID_ARG, "%s is NULL but requested by out_mask", what);
-        for (int i = 0; i < cnt; ++i) {
-            if (!src[i] || !aligned8(src[i]))
-                return fail(BLF_CCM_ERR_INVALID_ARG, "%s[%d] NULL or misaligned", what, i);
-            dst[i] = src[i];
-            vec = vec && aligned16(src[i]);
-        }
-        return BLF_CCM_OK;
+        return take_planes(src, dst, cnt, what);
     };
     if (out_mask & BLF_CCM_WRENCH)
-        if (int rc = take(wrench_planes, a.wrench, 6, "wrench_planes")) return rc;
+        if (int rc = take_out(wrench_planes, a.wrench, 6, "wrench_planes")) return rc;
     if (out_mask & BLF_CCM_AUTODYN)
-        if (int rc = take(autodyn_planes, a.autodyn, 6, "autodyn_planes")) return rc;
+        if (int rc = take_out(autodyn_planes, a.autodyn, 6, "autodyn_planes")) return rc;
     if (out_mask & BLF_CCM_REGRESSOR)
-        if (int rc = take(regressor_planes, a.reg, 12, "regressor_planes")) return rc;
+        if (int rc = take_out(regressor_planes, a.reg, 12, "regressor_planes")) return rc;
     if (out_mask & BLF_CCM_CTRL) {
-        if (!ctrl || !aligned8(ctrl)) return fail(BLF_CCM_ERR_INVALID_ARG, "ctrl NULL or misaligned");
-        a.ctrl = ctrl;
+        if (int rc = take_planes(&ctrl, &a.ctrl, 1, "ctrl")) return rc;
         a.ctrl_bulk = aligned16(ctrl) ? 1 : 0;
-        vec = vec && a.ctrl_bulk;
     }
     return BLF_CCM_OK;
 }
@@ -520,16 +488,14 @@ extern "C" int blf_ccm_eval_batch_soa(blf_ccm_handle* h, int64_t n, const double
     if (out_mask == 0 || out_mask > 15u) return fail(BLF_CCM_ERR_INVALID_ARG, "out_mask %u invalid", out_mask);
     if (n == 0) return BLF_CCM_OK;  // empty batch: nothing to read, nothing to write
     SoaArgs a;
-    bool vec = false;
     if (int rc = fill_soa_args(h, n, in_planes, param_planes, out_mask, out_mask, wrench_planes,
-                               autodyn_planes, ctrl, regressor_planes, a, vec))
+                               autodyn_planes, ctrl, regressor_planes, a))
         return rc;
     // planes only need 8-byte alignment; the dense 6x6 leaves by bulk copy when 16-byte aligned
     h->last_path = ((out_mask & BLF_CCM_CTRL) && !a.ctrl_bulk) ? BLF_CCM_PATH_DIRECT64 : BLF_CCM_PATH_BULK;
-    const bool vec2 = vec && h->tune_cpt == 2;
     cudaStream_t st = static_cast<cudaStream_t>(stream);
-    if (param_planes) return dispatch_mask<SoaLaunch, true>(out_mask, h, a, vec2, st);
-    return dispatch_mask<SoaLaunch, false>(out_mask, h, a, vec2, st);
+    if (param_planes) return dispatch_mask<SoaLaunch, true>(out_mask, h, a, st);
+    return dispatch_mask<SoaLaunch, false>(out_mask, h, a, st);
 }
 
 // ---- reverse mode of the wrench --------------------------------------------------------------------
@@ -575,34 +541,15 @@ extern "C" int blf_ccm_wrench_vjp_soa(blf_ccm_handle* h, int64_t n, const double
     a.uni[1] = h->width;
     a.uni[2] = h->spring;
     a.uni[3] = h->damper;
-    const unsigned live = vjp_live_planes(groups);
-    for (int i = 0; i < 30; ++i) {
-        if (!(live & (1u << i))) continue;
-        if (!in_planes[i])
-            return fail(BLF_CCM_ERR_INVALID_ARG, "in_planes[%d] is NULL but read for the requested gradients", i);
-        if (!aligned8(in_planes[i])) return fail(BLF_CCM_ERR_INVALID_ARG, "in_planes[%d] not 8-byte aligned", i);
-        a.in[i] = in_planes[i];
-    }
-    auto take = [&](const double* const* src, const double** dst, int cnt, bool nullable,
-                    const char* what) -> int {
-        for (int i = 0; i < cnt; ++i) {
-            if (!src[i] && nullable) continue;
-            if (!src[i] || !aligned8(src[i]))
-                return fail(BLF_CCM_ERR_INVALID_ARG, "%s[%d] NULL or misaligned", what, i);
-            dst[i] = src[i];
-        }
-        return BLF_CCM_OK;
-    };
+    if (int rc = take_planes(in_planes, a.in, 30, "in_planes", vjp_live_planes(groups))) return rc;
     if (param_planes)
-        if (int rc = take(param_planes, a.prm, 4, false, "param_planes")) return rc;
+        if (int rc = take_planes(param_planes, a.prm, 4, "param_planes")) return rc;
     if (grad_wrench_planes)
-        if (int rc = take(grad_wrench_planes, a.gw, 6, true, "grad_wrench_planes")) return rc;
+        if (int rc = take_planes(grad_wrench_planes, a.gw, 6, "grad_wrench_planes", ~0u, true)) return rc;
     if (grad_in_planes)
-        if (int rc = take(grad_in_planes, const_cast<const double**>(a.gin), 30, true, "grad_in_planes"))
-            return rc;
+        if (int rc = take_planes(grad_in_planes, a.gin, 30, "grad_in_planes", ~0u, true)) return rc;
     if (grad_param_planes)
-        if (int rc = take(grad_param_planes, const_cast<const double**>(a.gprm), 4, false, "grad_param_planes"))
-            return rc;
+        if (int rc = take_planes(grad_param_planes, a.gprm, 4, "grad_param_planes")) return rc;
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     if (param_planes) return dispatch_mask<VjpLaunch, true>(groups, h, a, st);
     return dispatch_mask<VjpLaunch, false>(groups, h, a, st);
@@ -618,19 +565,17 @@ struct AosLaunch {
             constexpr int threads = 64;
             const size_t smem = size_t(threads / 32) * AosSmem<MASK, HET>::bytes;
             auto k = ccm_aos_kernel<MASK, HET>;
-            int cap = 0;
-            if (int rc = persistent_blocks(h, k, threads, smem, &cap)) return rc;
+            if (int rc = prepare_kernel(h, k, threads, smem)) return rc;
             const long long tiles = (a.n + 31) / 32;
             const long long want = (tiles + threads / 32 - 1) / (threads / 32);
-            const int grid = static_cast<int>(std::min<long long>(want, cap));
+            const int grid = static_cast<int>(std::min<long long>(want, 0x7fffffff));   // grid-stride kernel
             CUDA_TRY(launch_pdl(h, k, grid, threads, smem, st, a));
         } else {
             constexpr int threads = 128;
             auto k = ccm_aos_scalar_kernel<MASK, HET>;
-            int cap = 0;
-            if (int rc = persistent_blocks(h, k, threads, 0, &cap)) return rc;
+            if (int rc = prepare_kernel(h, k, threads, 0)) return rc;
             const long long want = (a.n + threads - 1) / threads;
-            const int grid = static_cast<int>(std::min<long long>(want, cap));
+            const int grid = static_cast<int>(std::min<long long>(want, 0x7fffffff));   // grid-stride kernel
             k<<<grid, threads, 0, st>>>(a);
         }
         CUDA_TRY(cudaGetLastError());
@@ -1062,8 +1007,7 @@ struct CostLaunch {
         constexpr int threads = 128;
         const size_t smem = (OUT & M_CTRL) ? size_t(threads / 32) * 32 * 288 : 0;
         auto k = ccm_soa_kernel<OUT, HET, true>;
-        int cap = 0;
-        if (int rc = persistent_blocks(h, k, threads, smem, &cap)) return rc;
+        if (int rc = prepare_kernel(h, k, threads, smem)) return rc;
         const long long grid = (a.n + threads - 1) / threads;
         if (grid > 0x7fffffffLL) return fail(BLF_CCM_ERR_INVALID_ARG, "n too large for one launch");
         CUDA_TRY(launch_pdl(h, k, grid, threads, smem, st, a));
@@ -1109,10 +1053,9 @@ extern "C" int blf_ccm_rollout_cost_argmin_soa(blf_ccm_handle* h, int64_t n_roll
         return exchange_if_fused(h, best, stream);
     }
     SoaArgs a;
-    bool vec = false;
     if (int rc = fill_soa_args(h, n_rollouts * rollout_len, in_planes, param_planes, out_mask,
                                out_mask | BLF_CCM_WRENCH, wrench_planes, autodyn_planes, ctrl,
-                               nullptr, a, vec))
+                               nullptr, a))
         return rc;
     // per-(rollout, tile) partial sums: a rollout of length L intersects at most (L+62)/32 tiles
     const int slots = static_cast<int>((rollout_len + 62) / 32);
@@ -1315,16 +1258,14 @@ extern "C" int blf_rls_advance_batch(blf_ccm_handle* h, int64_t n, int p, int m,
     if (n == 0) return BLF_CCM_OK;
     if (!regressor_planes || !measurement_planes || !state_planes || !cov_planes)
         return fail(BLF_CCM_ERR_INVALID_ARG, "a plane-pointer array is NULL");
-    auto bad = [](const void* q) { return !q || !aligned8(q); };
     if (!rls_fast_path(p, m, lambda, host_measurement_cov)) {
         // any size / indefinite lambda R: the reference's own algorithm (pivoted LU)
-        std::vector<const double*> tabs;
-        for (int i = 0; i < m * p; ++i) tabs.push_back(regressor_planes[i]);
-        for (int i = 0; i < m; ++i) tabs.push_back(measurement_planes[i]);
-        for (int i = 0; i < p; ++i) tabs.push_back(state_planes[i]);
-        for (int i = 0; i < p * p; ++i) tabs.push_back(cov_planes[i]);
-        for (size_t i = 0; i < tabs.size(); ++i)
-            if (bad(tabs[i])) return fail(BLF_CCM_ERR_INVALID_ARG, "plane %zu NULL or misaligned", i);
+        std::vector<const double*> tabs(size_t(m * p + m + p + p * p));
+        const double** t = tabs.data();
+        if (int rc = take_planes(regressor_planes, t, m * p, "regressor_planes")) return rc;
+        if (int rc = take_planes(measurement_planes, t + m * p, m, "measurement_planes")) return rc;
+        if (int rc = take_planes(state_planes, t + m * p + m, p, "state_planes")) return rc;
+        if (int rc = take_planes(cov_planes, t + m * p + m + p, p * p, "cov_planes")) return rc;
         return rls_generic(h, n, p, m, tabs.data(), nullptr, nullptr, nullptr, nullptr, host_measurement_cov,
                            lambda, static_cast<cudaStream_t>(stream));
     }
@@ -1333,22 +1274,10 @@ extern "C" int blf_rls_advance_batch(blf_ccm_handle* h, int64_t n, int p, int m,
     a.n = n;
     a.lambda = lambda;
     for (int i = 0; i < m; ++i) a.w[i] = lambda * host_measurement_cov[i];
-    for (int i = 0; i < m * p; ++i) {
-        if (bad(regressor_planes[i])) return fail(BLF_CCM_ERR_INVALID_ARG, "regressor_planes[%d] NULL or misaligned", i);
-        a.Y[i] = regressor_planes[i];
-    }
-    for (int i = 0; i < m; ++i) {
-        if (bad(measurement_planes[i])) return fail(BLF_CCM_ERR_INVALID_ARG, "measurement_planes[%d] NULL or misaligned", i);
-        a.z[i] = measurement_planes[i];
-    }
-    for (int i = 0; i < p; ++i) {
-        if (bad(state_planes[i])) return fail(BLF_CCM_ERR_INVALID_ARG, "state_planes[%d] NULL or misaligned", i);
-        a.theta[i] = state_planes[i];
-    }
-    for (int i = 0; i < p * p; ++i) {
-        if (bad(cov_planes[i])) return fail(BLF_CCM_ERR_INVALID_ARG, "cov_planes[%d] NULL or misaligned", i);
-        a.cov[i] = cov_planes[i];
-    }
+    if (int rc = take_planes(regressor_planes, a.Y, m * p, "regressor_planes")) return rc;
+    if (int rc = take_planes(measurement_planes, a.z, m, "measurement_planes")) return rc;
+    if (int rc = take_planes(state_planes, a.theta, p, "state_planes")) return rc;
+    if (int rc = take_planes(cov_planes, a.cov, p * p, "cov_planes")) return rc;
     return rls_dispatch<false>(p, m, h, a, static_cast<cudaStream_t>(stream));
 }
 
@@ -1428,30 +1357,13 @@ extern "C" int blf_ccm_rls_advance_contacts(blf_ccm_handle* h, int64_t n,
     a.lambda = lambda;
     a.length = h->length;
     a.width = h->width;
-    auto bad = [](const void* q) { return !q || !aligned8(q); };
-    const unsigned live = live_planes(M_REGRESSOR);
-    for (int i = 0; i < 30; ++i) {
-        if (!(live & (1u << i))) continue;
-        if (bad(in_planes[i])) return fail(BLF_CCM_ERR_INVALID_ARG, "in_planes[%d] NULL or misaligned", i);
-        a.in[i] = in_planes[i];
-    }
-    for (int i = 0; i < 6; ++i) {
-        if (bad(measured_wrench_planes[i])) return fail(BLF_CCM_ERR_INVALID_ARG, "measured_wrench_planes[%d] NULL or misaligned", i);
-        a.z[i] = measured_wrench_planes[i];
-        a.w[i] = lambda * host_measurement_cov[i];
-    }
-    for (int i = 0; i < 2; ++i) {
-        if (bad(state_planes[i])) return fail(BLF_CCM_ERR_INVALID_ARG, "state_planes[%d] NULL or misaligned", i);
-        a.theta[i] = state_planes[i];
-        if (geometry_planes) {
-            if (bad(geometry_planes[i])) return fail(BLF_CCM_ERR_INVALID_ARG, "geometry_planes[%d] NULL or misaligned", i);
-            a.geom[i] = geometry_planes[i];
-        }
-    }
-    for (int i = 0; i < 4; ++i) {
-        if (bad(cov_planes[i])) return fail(BLF_CCM_ERR_INVALID_ARG, "cov_planes[%d] NULL or misaligned", i);
-        a.cov[i] = cov_planes[i];
-    }
+    for (int i = 0; i < 6; ++i) a.w[i] = lambda * host_measurement_cov[i];
+    if (int rc = take_planes(in_planes, a.in, 30, "in_planes", live_planes(M_REGRESSOR))) return rc;
+    if (int rc = take_planes(measured_wrench_planes, a.z, 6, "measured_wrench_planes")) return rc;
+    if (int rc = take_planes(state_planes, a.theta, 2, "state_planes")) return rc;
+    if (geometry_planes)
+        if (int rc = take_planes(geometry_planes, a.geom, 2, "geometry_planes")) return rc;
+    if (int rc = take_planes(cov_planes, a.cov, 4, "cov_planes")) return rc;
     const int threads = 128;
     const long long grid = (n + threads - 1) / threads;
     if (grid > 0x7fffffffLL) return fail(BLF_CCM_ERR_INVALID_ARG, "n too large for one launch");

@@ -6,8 +6,8 @@
 // whose warps march in lock-step (profiles/r01_variant_sweep.md).  HBM streams are touched once:
 //   SoA planes      coalesced 64-bit streaming loads / stores, one contact per lane (256 B per warp
 //                   request = two full 128 B lines; LDG.E.EF.64 / STG.E.EF.64).  A 128-bit,
-//                   two-contacts-per-lane variant (ccm_soa_vec2_kernel) is kept selectable: it is
-//                   slower on B200 because its 166 registers cap occupancy at 12 warps/SM;
+//                   two-contacts-per-lane variant was measured slower on B200 (its 166 registers
+//                   cap occupancy at 12 warps/SM) and removed (DESIGN §5);
 //   dense 6x6 ctrl  assembled per warp in shared memory, then ONE bulk async copy (TMA engine,
 //                   SASS UBLKCP) of tile*288 contiguous bytes;
 //   AoS structs     every input array arrives with a bulk async copy per tile signalled on a
@@ -46,54 +46,6 @@ struct SoaArgs {
     double* partials;          // [n_rollouts][slots] per-(rollout, tile) partial sums
     int slots;                 // max tiles one rollout can intersect
 };
-
-template <int CPT>
-struct Lanes {
-    double v[CPT];
-};
-
-// one plane, CPT consecutive contacts per lane
-template <int CPT>
-__device__ __forceinline__ Lanes<CPT> load_plane(const double* __restrict__ p, long long base,
-                                                 int lane, bool full, long long n)
-{
-    Lanes<CPT> r;
-    if (full) {
-        if constexpr (CPT == 2) {
-            const double2 t = __ldcs(reinterpret_cast<const double2*>(p + base) + lane);
-            r.v[0] = t.x;
-            r.v[1] = t.y;
-        } else {
-            r.v[0] = __ldcs(p + base + lane);
-        }
-    } else {
-#pragma unroll
-        for (int j = 0; j < CPT; ++j) {
-            const long long i = base + lane * CPT + j;
-            r.v[j] = i < n ? __ldcs(p + i) : 0.0;
-        }
-    }
-    return r;
-}
-
-template <int CPT>
-__device__ __forceinline__ void store_plane(double* __restrict__ p, long long base, int lane,
-                                            bool full, long long n, const double (&x)[CPT])
-{
-    if (full) {
-        if constexpr (CPT == 2) {
-            __stcs(reinterpret_cast<double2*>(p + base) + lane, make_double2(x[0], x[1]));
-        } else {
-            __stcs(p + base + lane, x[0]);
-        }
-    } else {
-#pragma unroll
-        for (int j = 0; j < CPT; ++j) {
-            const long long i = base + lane * CPT + j;
-            if (i < n) __stcs(p + i, x[j]);
-        }
-    }
-}
 
 // write the 12 non-structural entries of one dense 6x6 into its slot of the warp's tile
 __device__ __forceinline__ void stage_ctrl(double* slot, const Result& r)
@@ -172,37 +124,13 @@ ccm_soa_kernel(const __grid_constant__ SoaArgs a)
 
     // ---- every live plane in flight before the first use ---------------------------------------
     double x[30] = {};
-#pragma unroll
-    for (int pl = 0; pl < 30; ++pl)
-        if (LIVE & (1u << pl)) x[pl] = on ? __ldcs(a.in[pl] + i) : 0.0;
-    Prm q = a.uni;
-    if constexpr (HET) {
-        const double l = on ? __ldcs(a.prm[0] + i) : 0.0, w = on ? __ldcs(a.prm[1] + i) : 0.0;
-        const double k = on ? __ldcs(a.prm[2] + i) : 0.0, b = on ? __ldcs(a.prm[3] + i) : 0.0;
-        q = make_prm(l, w, k, b);
-    }
-
-    State s;
-    s.v = V3{x[0], x[1], x[2]};
-    s.w = V3{x[3], x[4], x[5]};
-    s.p = V3{x[6], x[7], x[8]};
-    s.e1 = V3{x[9], x[12], x[15]};
-    s.e2 = V3{x[10], x[13], x[16]};
-    s.R02 = x[11];
-    s.R12 = x[14];
-    s.R22 = x[17];
-    s.p0 = V3{x[18], x[19], x[20]};
-    s.n1 = V3{x[21], x[24], x[27]};
-    s.n2 = V3{x[22], x[25], x[28]};
+    load_live_planes<LIVE>(a.in, i, on, x);
+    const Prm q = load_params<HET>(a.prm, a.uni, i, on);
     Result r;
-    eval_contact<MASK>(s, q, r);
+    eval_contact<MASK>(state_from_planes(x), q, r);
 
     if (on) {
-        if constexpr ((OUT & M_WRENCH) != 0) {
-            __stcs(a.wrench[0] + i, r.force.x); __stcs(a.wrench[1] + i, r.force.y);
-            __stcs(a.wrench[2] + i, r.force.z); __stcs(a.wrench[3] + i, r.torque.x);
-            __stcs(a.wrench[4] + i, r.torque.y); __stcs(a.wrench[5] + i, r.torque.z);
-        }
+        if constexpr ((OUT & M_WRENCH) != 0) store_wrench(a.wrench, i, r);
         if constexpr ((OUT & M_AUTODYN) != 0) {
             __stcs(a.autodyn[0] + i, r.fhead.x); __stcs(a.autodyn[1] + i, r.fhead.y);
             __stcs(a.autodyn[2] + i, r.fhead.z); __stcs(a.autodyn[3] + i, r.ftail.x);
@@ -244,114 +172,6 @@ ccm_soa_kernel(const __grid_constant__ SoaArgs a)
     if constexpr ((OUT & M_CTRL) != 0) {
         // shared memory must stay valid until the bulk engine has read it
         if (a.ctrl_bulk && lane == 0) ptx::bulk_wait_read_all();
-    }
-}
-
-// 128-bit variant: two contacts per lane, double2 plane accesses, grid-stride over 64-contact tiles.
-template <unsigned MASK, bool HET>
-__global__ void __launch_bounds__(128, 3)
-ccm_soa_vec2_kernel(const __grid_constant__ SoaArgs a)
-{
-    constexpr int CPT = 2;
-    constexpr int TILE = kWarp * CPT;
-    constexpr unsigned LIVE = live_planes(MASK);
-    extern __shared__ __align__(128) unsigned char smem_raw[];
-
-    const int lane = threadIdx.x & 31;
-    const int warp = threadIdx.x >> 5;
-    const int warps_per_cta = blockDim.x >> 5;
-    double* ctile = reinterpret_cast<double*>(smem_raw) + static_cast<size_t>(warp) * TILE * 36;
-
-    if constexpr ((MASK & M_CTRL) != 0) {
-        // structural zeros: written once, never touched again
-        double2* z = reinterpret_cast<double2*>(ctile);
-        for (int i = lane; i < TILE * 18; i += kWarp) z[i] = make_double2(0.0, 0.0);
-        __syncwarp();
-    }
-
-    const long long ntiles = (a.n + TILE - 1) / TILE;
-    const long long wstride = static_cast<long long>(gridDim.x) * warps_per_cta;
-    for (long long t = static_cast<long long>(blockIdx.x) * warps_per_cta + warp; t < ntiles;
-         t += wstride) {
-        const long long base = t * TILE;
-        const bool full = base + TILE <= a.n;
-        const int cnt = full ? TILE : static_cast<int>(a.n - base);
-
-        // ---- all live planes in flight before the first use --------------------------------
-        Lanes<CPT> x[30] = {};
-#pragma unroll
-        for (int pl = 0; pl < 30; ++pl)
-            if (LIVE & (1u << pl)) x[pl] = load_plane<CPT>(a.in[pl], base, lane, full, a.n);
-        Lanes<CPT> pr[4] = {};
-        if constexpr (HET) {
-#pragma unroll
-            for (int pl = 0; pl < 4; ++pl) pr[pl] = load_plane<CPT>(a.prm[pl], base, lane, full, a.n);
-        }
-
-        Result r[CPT];
-#pragma unroll
-        for (int j = 0; j < CPT; ++j) {
-            State s;
-            s.v = V3{x[0].v[j], x[1].v[j], x[2].v[j]};
-            s.w = V3{x[3].v[j], x[4].v[j], x[5].v[j]};
-            s.p = V3{x[6].v[j], x[7].v[j], x[8].v[j]};
-            s.e1 = V3{x[9].v[j], x[12].v[j], x[15].v[j]};
-            s.e2 = V3{x[10].v[j], x[13].v[j], x[16].v[j]};
-            s.R02 = x[11].v[j];
-            s.R12 = x[14].v[j];
-            s.R22 = x[17].v[j];
-            s.p0 = V3{x[18].v[j], x[19].v[j], x[20].v[j]};
-            s.n1 = V3{x[21].v[j], x[24].v[j], x[27].v[j]};
-            s.n2 = V3{x[22].v[j], x[25].v[j], x[28].v[j]};
-            Prm q = a.uni;
-            if constexpr (HET) q = make_prm(pr[0].v[j], pr[1].v[j], pr[2].v[j], pr[3].v[j]);
-            eval_contact<MASK>(s, q, r[j]);
-        }
-
-        // ---- plane outputs: streaming stores ------------------------------------------------
-#define BLFCCM_STORE(ptr, field)                                        \
-    {                                                                   \
-        double o[CPT];                                                  \
-        _Pragma("unroll") for (int j = 0; j < CPT; ++j) o[j] = r[j].field; \
-        store_plane<CPT>(ptr, base, lane, full, a.n, o);                \
-    }
-        if constexpr ((MASK & M_WRENCH) != 0) {
-            BLFCCM_STORE(a.wrench[0], force.x) BLFCCM_STORE(a.wrench[1], force.y)
-            BLFCCM_STORE(a.wrench[2], force.z) BLFCCM_STORE(a.wrench[3], torque.x)
-            BLFCCM_STORE(a.wrench[4], torque.y) BLFCCM_STORE(a.wrench[5], torque.z)
-        }
-        if constexpr ((MASK & M_AUTODYN) != 0) {
-            BLFCCM_STORE(a.autodyn[0], fhead.x) BLFCCM_STORE(a.autodyn[1], fhead.y)
-            BLFCCM_STORE(a.autodyn[2], fhead.z) BLFCCM_STORE(a.autodyn[3], ftail.x)
-            BLFCCM_STORE(a.autodyn[4], ftail.y) BLFCCM_STORE(a.autodyn[5], ftail.z)
-        }
-        if constexpr ((MASK & M_REGRESSOR) != 0) {
-            // row-major 6x2: plane 2*row + col, col 0 = spring, col 1 = damper
-            BLFCCM_STORE(a.reg[0], y_fk.x) BLFCCM_STORE(a.reg[1], y_fb.x)
-            BLFCCM_STORE(a.reg[2], y_fk.y) BLFCCM_STORE(a.reg[3], y_fb.y)
-            BLFCCM_STORE(a.reg[4], y_fk.z) BLFCCM_STORE(a.reg[5], y_fb.z)
-            BLFCCM_STORE(a.reg[6], y_tk.x) BLFCCM_STORE(a.reg[7], y_tb.x)
-            BLFCCM_STORE(a.reg[8], y_tk.y) BLFCCM_STORE(a.reg[9], y_tb.y)
-            BLFCCM_STORE(a.reg[10], y_tk.z) BLFCCM_STORE(a.reg[11], y_tb.z)
-        }
-#undef BLFCCM_STORE
-
-        // ---- dense 6x6: shared-memory assembly + one bulk store per tile -------------------
-        if constexpr ((MASK & M_CTRL) != 0) {
-            if (a.ctrl_bulk) {
-                if (lane == 0) ptx::bulk_wait_read_all();  // previous tile left shared memory
-            }
-            __syncwarp();
-#pragma unroll
-            for (int j = 0; j < CPT; ++j) {
-                const int li = lane * CPT + j;
-                if (li < cnt) stage_ctrl(ctile + li * 36, r[j]);
-            }
-            flush_ctrl_tile(a.ctrl, ctile, base, cnt, lane, a.ctrl_bulk != 0);
-        }
-    }
-    if constexpr ((MASK & M_CTRL) != 0) {
-        if (a.ctrl_bulk && lane == 0) ptx::bulk_wait_all();
     }
 }
 
@@ -798,9 +618,7 @@ ccm_wrench_vjp_kernel(const __grid_constant__ VjpArgs a)
     ptx::grid_dep_wait();
 
     double x[30] = {};
-#pragma unroll
-    for (int pl = 0; pl < 30; ++pl)
-        if (LIVE & (1u << pl)) x[pl] = on ? __ldcs(a.in[pl] + i) : 0.0;
+    load_live_planes<LIVE>(a.in, i, on, x);
     double gw[6];
 #pragma unroll
     for (int j = 0; j < 6; ++j) gw[j] = (on && a.gw[j]) ? __ldcs(a.gw[j] + i) : 0.0;
@@ -813,20 +631,8 @@ ccm_wrench_vjp_kernel(const __grid_constant__ VjpArgs a)
     }
     const Prm q = make_prm(l, w, k, b);
 
-    State s;
-    s.v = V3{x[0], x[1], x[2]};
-    s.w = V3{x[3], x[4], x[5]};
-    s.p = V3{x[6], x[7], x[8]};
-    s.e1 = V3{x[9], x[12], x[15]};
-    s.e2 = V3{x[10], x[13], x[16]};
-    s.R02 = 0.0;
-    s.R12 = 0.0;
-    s.R22 = x[17];
-    s.p0 = V3{x[18], x[19], x[20]};
-    s.n1 = V3{x[21], x[24], x[27]};
-    s.n2 = V3{x[22], x[25], x[28]};
     VjpOut g;
-    vjp_wrench<GROUPS>(s, q, l, w, V3{gw[0], gw[1], gw[2]}, V3{gw[3], gw[4], gw[5]}, g);
+    vjp_wrench<GROUPS>(state_from_planes(x), q, l, w, V3{gw[0], gw[1], gw[2]}, V3{gw[3], gw[4], gw[5]}, g);
     if (!on) return;
 
     auto put = [&](int pl, double val) {

@@ -172,6 +172,59 @@ __host__ __device__ constexpr unsigned live_planes(unsigned mask)
     return all;
 }
 
+// ---- reading and writing the SoA contact state --------------------------------------------------
+// 30 input planes: twist (0-5), pose p | R row-major (6-17), null pose p0 | R0 row-major (18-29);
+// 4 parameter planes: length, width, spring, damper.  Lanes past the end (!on) read zeros.
+
+// The live planes into x (x zero-initialised by the caller: dead planes stay +0.0).  This exact
+// form keeps every caller's machine code unchanged; folding the LIVE test into the condition does not.
+template <unsigned LIVE>
+__device__ __forceinline__ void load_live_planes(const double* const (&in)[30], long long i, bool on,
+                                                 double (&x)[30])
+{
+#pragma unroll
+    for (int pl = 0; pl < 30; ++pl)
+        if (LIVE & (1u << pl)) x[pl] = on ? __ldcs(in[pl] + i) : 0.0;
+}
+
+__device__ __forceinline__ State state_from_planes(const double (&x)[30])
+{
+    State s;
+    s.v = V3{x[0], x[1], x[2]};
+    s.w = V3{x[3], x[4], x[5]};
+    s.p = V3{x[6], x[7], x[8]};
+    s.e1 = V3{x[9], x[12], x[15]};
+    s.e2 = V3{x[10], x[13], x[16]};
+    s.R02 = x[11];
+    s.R12 = x[14];
+    s.R22 = x[17];
+    s.p0 = V3{x[18], x[19], x[20]};
+    s.n1 = V3{x[21], x[24], x[27]};
+    s.n2 = V3{x[22], x[25], x[28]};
+    return s;
+}
+
+// the uniform parameters, or (HET) this contact's parameter planes
+template <bool HET>
+__device__ __forceinline__ Prm load_params(const double* const (&prm)[4], const Prm& uni, long long i, bool on)
+{
+    Prm q = uni;
+    if constexpr (HET) {
+        const double l = on ? __ldcs(prm[0] + i) : 0.0, w = on ? __ldcs(prm[1] + i) : 0.0;
+        const double k = on ? __ldcs(prm[2] + i) : 0.0, b = on ? __ldcs(prm[3] + i) : 0.0;
+        q = make_prm(l, w, k, b);
+    }
+    return q;
+}
+
+// force | torque into six planes
+__device__ __forceinline__ void store_wrench(double* const (&wrench)[6], long long i, const Result& r)
+{
+    __stcs(wrench[0] + i, r.force.x); __stcs(wrench[1] + i, r.force.y);
+    __stcs(wrench[2] + i, r.force.z); __stcs(wrench[3] + i, r.torque.x);
+    __stcs(wrench[4] + i, r.torque.y); __stcs(wrench[5] + i, r.torque.z);
+}
+
 // ------------------------------------------------------------------------------------------------
 // Reverse mode of the wrench: gbar^T d(wrench)/d(inputs) for a cotangent gbar = (gF, gT).
 // With ac = |R22|, alpha = ac A, beta = ac A/12, sd = k (p0 - p) - b v, u_i = e_i x (e_i x w),

@@ -422,9 +422,7 @@ ccm_rls_kernel(const __grid_constant__ CcmRlsArgs a)
     const long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
     if (i >= a.n) return;
     double x[30] = {};
-#pragma unroll
-    for (int pl = 0; pl < 30; ++pl)
-        if (LIVE & (1u << pl)) x[pl] = __ldcs(a.in[pl] + i);
+    load_live_planes<LIVE>(a.in, i, true, x);
     double z[6], r[6], th[2], C[2][2];
 #pragma unroll
     for (int q = 0; q < 6; ++q) {
@@ -440,19 +438,8 @@ ccm_rls_kernel(const __grid_constant__ CcmRlsArgs a)
         L = __ldcs(a.geom[0] + i);
         W = __ldcs(a.geom[1] + i);
     }
-    State s;
-    s.v = V3{x[0], x[1], x[2]};
-    s.w = V3{x[3], x[4], x[5]};
-    s.p = V3{x[6], x[7], x[8]};
-    s.e1 = V3{x[9], x[12], x[15]};
-    s.e2 = V3{x[10], x[13], x[16]};
-    s.R02 = 0.0; s.R12 = 0.0;
-    s.R22 = x[17];
-    s.p0 = V3{x[18], x[19], x[20]};
-    s.n1 = V3{x[21], x[24], x[27]};
-    s.n2 = V3{x[22], x[25], x[28]};
     Result res;
-    eval_contact<M_REGRESSOR>(s, make_prm(L, W, 0.0, 0.0), res);
+    eval_contact<M_REGRESSOR>(state_from_planes(x), make_prm(L, W, 0.0, 0.0), res);
     const double Y[6][2] = {{res.y_fk.x, res.y_fb.x}, {res.y_fk.y, res.y_fb.y}, {res.y_fk.z, res.y_fb.z},
                             {res.y_tk.x, res.y_tb.x}, {res.y_tk.y, res.y_tb.y}, {res.y_tk.z, res.y_tb.z}};
     rls_advance<2, 6>(Y, z, r, a.lambda, th, C);

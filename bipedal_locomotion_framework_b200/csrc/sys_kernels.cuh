@@ -1592,33 +1592,11 @@ ccm_genforce_kernel(const __grid_constant__ GenForceArgs a)
     const bool on = lane < ncont;
     const long long i = c0 + lane;
     double x[30] = {};
-#pragma unroll
-    for (int pl = 0; pl < 30; ++pl)
-        if (LIVE & (1u << pl)) x[pl] = on ? __ldcs(a.in[pl] + i) : 0.0;
-    Prm q = a.uni;
-    if constexpr (HET) {
-        const double l = on ? __ldcs(a.prm[0] + i) : 0.0, w = on ? __ldcs(a.prm[1] + i) : 0.0;
-        const double k = on ? __ldcs(a.prm[2] + i) : 0.0, b = on ? __ldcs(a.prm[3] + i) : 0.0;
-        q = make_prm(l, w, k, b);
-    }
-    State st;
-    st.v = V3{x[0], x[1], x[2]};
-    st.w = V3{x[3], x[4], x[5]};
-    st.p = V3{x[6], x[7], x[8]};
-    st.e1 = V3{x[9], x[12], x[15]};
-    st.e2 = V3{x[10], x[13], x[16]};
-    st.R02 = 0.0; st.R12 = 0.0;
-    st.R22 = x[17];
-    st.p0 = V3{x[18], x[19], x[20]};
-    st.n1 = V3{x[21], x[24], x[27]};
-    st.n2 = V3{x[22], x[25], x[28]};
+    load_live_planes<LIVE>(a.in, i, on, x);
+    const Prm q = load_params<HET>(a.prm, a.uni, i, on);
     Result r;
-    eval_contact<M_WRENCH>(st, q, r);
-    if (a.want_wrench && on) {
-        __stcs(a.wrench[0] + i, r.force.x); __stcs(a.wrench[1] + i, r.force.y);
-        __stcs(a.wrench[2] + i, r.force.z); __stcs(a.wrench[3] + i, r.torque.x);
-        __stcs(a.wrench[4] + i, r.torque.y); __stcs(a.wrench[5] + i, r.torque.z);
-    }
+    eval_contact<M_WRENCH>(state_from_planes(x), q, r);
+    if (a.want_wrench && on) store_wrench(a.wrench, i, r);
     {
         double2* o = reinterpret_cast<double2*>(wsm) + lane * 3;
         o[0] = make_double2(r.force.x, r.force.y);
@@ -1795,33 +1773,11 @@ ccm_genforce_packed_kernel(const __grid_constant__ GenForceArgs a)
     const bool on = lane < ncont;
     const long long i = c0 + lane;
     double x[30] = {};
-#pragma unroll
-    for (int pl = 0; pl < 30; ++pl)
-        if (LIVE & (1u << pl)) x[pl] = on ? __ldcs(a.in[pl] + i) : 0.0;
-    Prm q = a.uni;
-    if constexpr (HET) {
-        const double l = on ? __ldcs(a.prm[0] + i) : 0.0, w = on ? __ldcs(a.prm[1] + i) : 0.0;
-        const double k = on ? __ldcs(a.prm[2] + i) : 0.0, b = on ? __ldcs(a.prm[3] + i) : 0.0;
-        q = make_prm(l, w, k, b);
-    }
-    State st;
-    st.v = V3{x[0], x[1], x[2]};
-    st.w = V3{x[3], x[4], x[5]};
-    st.p = V3{x[6], x[7], x[8]};
-    st.e1 = V3{x[9], x[12], x[15]};
-    st.e2 = V3{x[10], x[13], x[16]};
-    st.R02 = 0.0; st.R12 = 0.0;
-    st.R22 = x[17];
-    st.p0 = V3{x[18], x[19], x[20]};
-    st.n1 = V3{x[21], x[24], x[27]};
-    st.n2 = V3{x[22], x[25], x[28]};
+    load_live_planes<LIVE>(a.in, i, on, x);
+    const Prm q = load_params<HET>(a.prm, a.uni, i, on);
     Result r;
-    eval_contact<M_WRENCH>(st, q, r);
-    if (a.want_wrench && on) {
-        __stcs(a.wrench[0] + i, r.force.x); __stcs(a.wrench[1] + i, r.force.y);
-        __stcs(a.wrench[2] + i, r.force.z); __stcs(a.wrench[3] + i, r.torque.x);
-        __stcs(a.wrench[4] + i, r.torque.y); __stcs(a.wrench[5] + i, r.torque.z);
-    }
+    eval_contact<M_WRENCH>(state_from_planes(x), q, r);
+    if (a.want_wrench && on) store_wrench(a.wrench, i, r);
     {
         double2* o = reinterpret_cast<double2*>(wsm) + lane * 3;
         o[0] = make_double2(r.force.x, r.force.y);

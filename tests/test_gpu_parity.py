@@ -256,31 +256,6 @@ def test_eight_byte_aligned_buffers_take_the_checked_64bit_path(torch, batch, or
     _check(got, ref, FULL, f"unaligned/{layout}")
 
 
-def test_128bit_two_contacts_per_lane_variant(torch, oracle, monkeypatch):
-    """The selectable 128-bit SoA kernel (BLF_CCM_TUNE_CPT=2), persistent and one-tile-per-warp."""
-    from bipedal_locomotion_framework_b200.contact_models import ContinuousContactModelBatch
-    n = 100000 + 17
-    st = syn.make_states(n + 1, seed=23, heterogeneous=True)
-    st = {k: (v[:n] if isinstance(v, np.ndarray) else v) for k, v in st.items()}
-    ref = oracle.eval_batch_states(st, mask=FULL | R, nthreads=NTHREADS)
-    big = torch.empty((30, n + 1), dtype=torch.float64, device="cuda")  # even pitch: rows 16-B aligned
-    planes = big[:, :n]
-    planes.copy_(_dev(torch, syn.aos_to_planes(st["twists"], st["poses"], st["null_poses"])))
-    pbig = torch.empty((4, n + 1), dtype=torch.float64, device="cuda")
-    prm = pbig[:, :n]
-    prm.copy_(_dev(torch, st["params"].T))
-    for blocks in ("0", "2"):
-        monkeypatch.setenv("BLF_CCM_TUNE_CPT", "2")
-        monkeypatch.setenv("BLF_CCM_TUNE_BLOCKS_PER_SM", blocks)
-        b = ContinuousContactModelBatch(0)
-        b.set_uniform_params(*syn.REFERENCE_TEST_PARAMS)
-        out = {k: torch.empty((c, n + 1), dtype=torch.float64, device="cuda")[:, :n]
-               for k, c in (("wrench", 6), ("autodyn", 6), ("regressor", 12))}
-        out["ctrl"] = torch.empty((n, 36), dtype=torch.float64, device="cuda")
-        b.evaluate_soa(planes, prm, FULL | R, out=out)
-        _check(_soa_out_to_aos(out), ref, FULL | R, f"vec2 blocks={blocks}")
-
-
 def test_uninitialised_handle_is_an_error(torch):
     from bipedal_locomotion_framework_b200 import _capi
     from bipedal_locomotion_framework_b200.contact_models import ContinuousContactModelBatch

@@ -42,8 +42,6 @@ def row(name, ms, n, bytes_per):
 
 
 def make_batch(**env):
-    for k in ("BLF_CCM_TUNE_CPT", "BLF_CCM_TUNE_BLOCKS_PER_SM"):
-        os.environ.pop(k, None)
     for k, v in env.items():
         os.environ[k] = str(v)
     b = ContinuousContactModelBatch(0)
@@ -289,16 +287,11 @@ def main():
                for k in ("twists", "poses", "null_poses")]
         prm_aos = prm.T.contiguous()
         print(f"\n=== n = {n} ({label}); peak {PEAK} GB/s ===")
-        for cpt, bps in ((1, 0), (2, 0), (2, 3), (2, 2)):
-            b = make_batch(BLF_CCM_TUNE_CPT=cpt, BLF_CCM_TUNE_BLOCKS_PER_SM=bps)
-            outs = [b.alloc_soa_outputs(n, FULL) for _ in range(NS)]
-            cl = [b.prepare_soa(planes[j], None, FULL, out=outs[j])[0] for j in range(NS)]
-            ms = timeit(lambda i: cl[i % NS]())
-            row(f"soa full uniform contacts/lane={cpt} {'persistent %d CTA/SM' % bps if bps else 'one tile/warp'}",
-                ms, n, 600)
-            del outs
         b = make_batch()
         outs = [b.alloc_soa_outputs(n, FULL) for _ in range(NS)]
+        cl = [b.prepare_soa(planes[j], None, FULL, out=outs[j])[0] for j in range(NS)]
+        ms = timeit(lambda i: cl[i % NS]())
+        row("soa full uniform", ms, n, 600)
         cl = [b.prepare_soa(planes[j], prm, FULL, out=outs[j])[0] for j in range(NS)]
         ms = timeit(lambda i: cl[i % NS]())
         row("soa full heterogeneous", ms, n, 632)
@@ -312,20 +305,13 @@ def main():
         row(f"rollout({rl}) cost only (25 planes in)", ms, n, 200)
         del outs
         outs = [b.alloc_soa_outputs(n, WRENCH) for _ in range(NS)]
-        for cpt in (1, 2):
-            b2 = make_batch(BLF_CCM_TUNE_CPT=cpt)
-            cl = [b2.prepare_soa(planes[j], None, WRENCH, out=outs[j])[0] for j in range(NS)]
-            ms = timeit(lambda i: cl[i % NS]())
-            row(f"soa wrench-only uniform contacts/lane={cpt}", ms, n, 248)
+        cl = [b.prepare_soa(planes[j], None, WRENCH, out=outs[j])[0] for j in range(NS)]
+        ms = timeit(lambda i: cl[i % NS]())
+        row("soa wrench-only uniform", ms, n, 248)
         del outs
-        for bps in (0, 2):
-            b3 = make_batch(BLF_CCM_TUNE_BLOCKS_PER_SM=bps)
-            outs = [b3.alloc_aos_outputs(n, FULL) for _ in range(2)]
-            ms = timeit(lambda i: b3.evaluate_aos(aos[0], aos[1], aos[2], None, FULL, out=outs[i % 2]))
-            row(f"aos full uniform {'persistent %d CTA/SM' % bps if bps else 'one tile/warp'} (624 B touched)", ms, n, 600)
-            del outs
-        b = make_batch()
         outs = [b.alloc_aos_outputs(n, FULL) for _ in range(2)]
+        ms = timeit(lambda i: b.evaluate_aos(aos[0], aos[1], aos[2], None, FULL, out=outs[i % 2]))
+        row("aos full uniform (624 B touched)", ms, n, 600)
         ms = timeit(lambda i: b.evaluate_aos(aos[0], aos[1], aos[2], prm_aos, FULL, out=outs[i % 2]))
         row("aos full heterogeneous", ms, n, 632)
         del outs
