@@ -105,6 +105,59 @@ def closed_form(v, w, p, R, p0, R0, L, W, k, b, zero):
     return {"wrench": force + torque, "autodyn": head + tail, "ctrl": ctrl, "regressor": reg}
 
 
+def exact_surface_point(twist, pose, null_pose, params, x, y):
+    """getForceAtPoint / getTorqueGeneratedAtPoint (ContinuousContactModel.cpp:185-219) of one
+    point q = (x, y, 0) as exact Fractions: (force[3], torque[3]).
+
+    Zero outside |x| <= length/2, |y| <= width/2 (the reference tests with a strict >, so the
+    boundary is inside); else f = k((p0 - p) + (R0 - R) q) - b(v + w x R q) and tau = R q x f.
+    params = (length, width, spring, damper)."""
+    fr = lambda xs: [F(float(v)) for v in xs]
+    L, W, k, b = fr(params)
+    X, Y = F(float(x)), F(float(y))
+    if abs(X) > L / 2 or abs(Y) > W / 2:
+        return [F(0)] * 3, [F(0)] * 3
+    v, w, p, R = fr(twist[0:3]), fr(twist[3:6]), fr(pose[0:3]), fr(pose[3:12])
+    p0, R0 = fr(null_pose[0:3]), fr(null_pose[3:12])
+    rq = [R[3 * i] * X + R[3 * i + 1] * Y for i in range(3)]
+    r0q = [R0[3 * i] * X + R0[3 * i + 1] * Y for i in range(3)]
+    wrq = _cross(w, rq)
+    f = [k * ((p0[i] - p[i]) + (r0q[i] - rq[i])) - b * (v[i] + wrq[i]) for i in range(3)]
+    return f, _cross(rq, f)
+
+
+def surface_edge_points(length, width):
+    """(49, 2) points on and around the rectangle's rim: every pair of x in {+-L/2, the next double
+    outside each, +-0.0, an interior value} and the same for y -- edges, corners, signed zeros."""
+    hl, hw = abs(float(length)) / 2, abs(float(width)) / 2
+    xs = [hl, -hl, np.nextafter(hl, np.inf), np.nextafter(-hl, -np.inf), 0.0, -0.0, 0.3 * hl]
+    ys = [hw, -hw, np.nextafter(hw, np.inf), np.nextafter(-hw, -np.inf), 0.0, -0.0, -0.7 * hw]
+    return np.array([[x, y] for x in xs for y in ys], dtype=np.float64)
+
+
+def surface_points_f64(twist, pose, null_pose, params, xy):
+    """The same closed form in plain float64 numpy for many points xy (m, 2), with the operand
+    magnitudes that bound its rounding error: returns force (m, 3), torque (m, 3),
+    fmag = k(|p0 - p| + |R0 q| + |R q|) + b(|v| + |w||R q|) and tmag = fmag |R q| (both (m,))."""
+    twist, pose, null_pose = (np.asarray(a, dtype=np.float64) for a in (twist, pose, null_pose))
+    L, W, k, b = (float(v) for v in params)
+    xy = np.asarray(xy, dtype=np.float64).reshape(-1, 2)
+    x, y = xy[:, 0:1], xy[:, 1:2]
+    R, R0 = pose[3:12].reshape(3, 3), null_pose[3:12].reshape(3, 3)
+    v, w, dp = twist[0:3], twist[3:6], null_pose[0:3] - pose[0:3]
+    rq = x * R[:, 0] + y * R[:, 1]
+    r0q = x * R0[:, 0] + y * R0[:, 1]
+    f = k * (dp + (r0q - rq)) - b * (v + np.cross(w, rq))
+    t = np.cross(rq, f)
+    inside = ~((np.abs(x[:, 0]) > L / 2) | (np.abs(y[:, 0]) > W / 2))
+    f[~inside] = 0.0
+    t[~inside] = 0.0
+    nrq = np.linalg.norm(rq, axis=1)
+    fmag = (abs(k) * (np.linalg.norm(dp) + np.linalg.norm(r0q, axis=1) + nrq)
+            + abs(b) * (np.linalg.norm(v) + np.linalg.norm(w) * nrq))
+    return f, t, fmag, fmag * nrq
+
+
 def exact_eval_rounded(twist, pose, null_pose, params):
     ex = exact_eval(twist, pose, null_pose, params)
     return {k: np.array([float(x) for x in vals]) for k, vals in ex.items()}

@@ -77,6 +77,22 @@ def exact_euler_step(rho, dT, twist, pos, rot):
     return (np.array([float(x) for x in pd]), fl(Rd), np.array([float(x) for x in pn]), fl(Rn))
 
 
+def mp_trajectory(rho, dts, twist, pos, rot, digits=50):
+    """ForwardEuler steps of sizes dts (constant twist) at `digits` significant digits, rounded once
+    at the end: (pos (3,), rot (3, 3)) as doubles."""
+    import mpmath as mp
+    with mp.workdps(digits):
+        m = lambda x: mp.mpf(float(x))
+        zero, one = mp.mpf(0), mp.mpf(1)
+        v, w = [m(x) for x in twist[:3]], [m(x) for x in twist[3:6]]
+        p = [m(x) for x in pos]
+        R = [[m(x) for x in row] for row in np.asarray(rot).reshape(3, 3)]
+        rho_ = m(rho)
+        for dT in dts:
+            p, R = euler_step(rho_, m(dT), v, w, p, R, zero, one)
+        return np.array([float(x) for x in p]), np.array([[float(x) for x in row] for row in R])
+
+
 def mp_rollout(n_rollouts, feet, horizon, dT, rho, twist_planes, pos, rot, null, params,
                wrench_ref, weights, digits=80):
     """80-digit rollout.  twist_planes (6, horizon*chains) time-major, pos (3,chains), rot
