@@ -29,7 +29,7 @@ SYMBOLS = [
     "blf_ccm_copy_h2d", "blf_ccm_copy_d2h", "blf_ccm_stream_synchronize",
     "blf_rls_advance_batch", "blf_rls_advance_host", "blf_ccm_rls_advance_contacts",
     "blf_sys_kinematics_euler_step_soa", "blf_sys_kinematics_dynamics_host", "blf_sys_kinematics_dynamics",
-    "blf_sys_kinematics_integrate_host", "blf_ccm_rollout_integrate_cost",
+    "blf_sys_kinematics_integrate_host", "blf_ccm_rollout_integrate_cost", "blf_ccm_rollout_cost_vjp",
     "blf_ccm_generalized_force_soa", "blf_ccm_rollout_integrate_cost_host",
     "blf_sys_mass_matrix_solve", "blf_sys_floating_base_acceleration", "blf_sys_floating_base_euler_step",
     "blf_ccm_p2p_mailbox_create", "blf_ccm_p2p_mailbox_connect", "blf_ccm_argmin_exchange_p2p",
@@ -92,6 +92,8 @@ def lib():
                                                     vp, vp]
     L.blf_ccm_rollout_integrate_cost.argtypes = [vp, i64, ci, ci, dbl, dbl, vp, vp, vp, vp, vp, u32,
                                                  vp, vp, vp, vp, vp, vp, vp, i64, vp, vp, vp]
+    L.blf_ccm_rollout_cost_vjp.argtypes = [vp, i64, ci, ci, dbl, dbl, vp, vp, vp, vp, vp, vp, vp, vp,
+                                           vp, vp, vp, vp, vp, vp]
     L.blf_ccm_rollout_integrate_cost_host.argtypes = [vp, i64, ci, ci, dbl, dbl, vp, vp, vp, vp, vp,
                                                       vp, vp, vp, vp, vp]
     L.blf_ccm_generalized_force_soa.argtypes = [vp, i64, ci, ci, vp, vp, vp, vp, vp, vp, vp]

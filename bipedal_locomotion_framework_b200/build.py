@@ -88,6 +88,7 @@ CPP_TESTS = {
     "FloatingBaseSystemDynamicsUnitTests": "FloatingBaseSystemDynamicsTest.cpp",   # needs a GPU
     "ApiConformanceUnitTests": "ApiConformanceTest.cpp",                   # compile-time signature checks
     "ContactWrenchGradientUnitTests": "ContactWrenchGradientTest.cpp",     # needs a GPU
+    "RolloutGradientUnitTests": "RolloutGradientTest.cpp",                 # needs a GPU
 }
 CXX_FLAGS = ["-std=c++17", "-O2", "-fPIC", "-Wall", "-Wextra"]
 

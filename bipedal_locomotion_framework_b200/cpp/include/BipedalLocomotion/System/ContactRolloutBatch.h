@@ -66,6 +66,28 @@ public:
                  double forceWeight, double torqueWeight, Result& result);
 
     /**
+     * Reverse mode of the rollouts' cost (blf_ccm_rollout_cost_vjp; no reference counterpart): for
+     * the cotangents gradCost (device, nRollouts) of the costs `rollout` computes from the same
+     * inputs, writes gradCost^T dcost/d(input) into the requested outputs -- twistGradient 6 planes
+     * of horizon*chains (time-major), positionGradient + rotationGradient 3 + 9 planes (both or
+     * neither), nullPoseGradient 12, parameterGradient 4 planes of chains (each chain's share).
+     * nullptr = not requested; at least one must be given.  Outputs must not alias inputs.
+     */
+    bool rolloutCostGradient(std::size_t nRollouts, int feet, int horizon, double dT, double rho,
+                             const GenericContainer::DeviceSoA& twists,
+                             const GenericContainer::DeviceSoA& positions,
+                             const GenericContainer::DeviceSoA& rotations,
+                             const GenericContainer::DeviceSoA& nullPoses,
+                             const GenericContainer::DeviceSoA* parameters,
+                             const iDynTree::Wrench& referenceWrench, double forceWeight,
+                             double torqueWeight, const double* gradCost,
+                             GenericContainer::DeviceSoA* twistGradient,
+                             GenericContainer::DeviceSoA* positionGradient,
+                             GenericContainer::DeviceSoA* rotationGradient,
+                             GenericContainer::DeviceSoA* nullPoseGradient,
+                             GenericContainer::DeviceSoA* parameterGradient, void* stream = nullptr);
+
+    /**
      * Cost-only rollouts with every plane in HOST memory (blf_ccm_rollout_integrate_cost_host):
      * twistPlanes[6] of horizon*chains doubles (time-major), positionPlanes[3], rotationPlanes[9],
      * nullPosePlanes[12] (third rotation column may be null) and optional parameterPlanes[4] of

@@ -1,6 +1,7 @@
 /**
  * @file ContactRolloutBatch.cpp
- * Thin C++17 layer over blf_sys_kinematics_euler_step_soa, blf_ccm_rollout_integrate_cost and
+ * Thin C++17 layer over blf_sys_kinematics_euler_step_soa, blf_ccm_rollout_integrate_cost,
+ * blf_ccm_rollout_cost_vjp and
  * blf_ccm_generalized_force_soa.
  */
 #include <iostream>
@@ -90,6 +91,43 @@ bool ContactRolloutBatch::rollout(std::size_t nRollouts, int feet, int horizon, 
                       finalRotations ? finalRotations->planePointers() : nullptr, referenceWrench.data(),
                       weights, indexBase, costs, best, stream),
                   "rollout");
+}
+
+bool ContactRolloutBatch::rolloutCostGradient(std::size_t nRollouts, int feet, int horizon, double dT,
+                                              double rho, const DeviceSoA& twists, const DeviceSoA& positions,
+                                              const DeviceSoA& rotations, const DeviceSoA& nullPoses,
+                                              const DeviceSoA* parameters, const iDynTree::Wrench& referenceWrench,
+                                              double forceWeight, double torqueWeight, const double* gradCost,
+                                              DeviceSoA* twistGradient, DeviceSoA* positionGradient,
+                                              DeviceSoA* rotationGradient, DeviceSoA* nullPoseGradient,
+                                              DeviceSoA* parameterGradient, void* stream)
+{
+    const char* where = "rolloutCostGradient";
+    if (m_device == nullptr) return report(BLF_CCM_ERR_INVALID_HANDLE, where);
+    if (feet < 1 || horizon < 1)
+    {
+        std::cerr << "[ContactRolloutBatch::rolloutCostGradient] feet and horizon must be positive." << std::endl;
+        return false;
+    }
+    const std::size_t chains = nRollouts * static_cast<std::size_t>(feet);
+    const std::size_t steps = chains * static_cast<std::size_t>(horizon);
+    if (!planes(twists, 6, steps, "twists", where) || !planes(positions, 3, chains, "positions", where)
+        || !planes(rotations, 9, chains, "rotations", where) || !planes(nullPoses, 12, chains, "nullPoses", where)
+        || (twistGradient && !planes(*twistGradient, 6, steps, "twistGradient", where))
+        || (positionGradient && !planes(*positionGradient, 3, chains, "positionGradient", where))
+        || (rotationGradient && !planes(*rotationGradient, 9, chains, "rotationGradient", where))
+        || (nullPoseGradient && !planes(*nullPoseGradient, 12, chains, "nullPoseGradient", where))
+        || (parameterGradient && !planes(*parameterGradient, 4, chains, "parameterGradient", where)))
+        return false;
+    const double weights[2] = {forceWeight, torqueWeight};
+    auto out = [](DeviceSoA* s) { return s ? s->planePointers() : nullptr; };
+    return report(blf_ccm_rollout_cost_vjp(
+                      raw(m_device), static_cast<std::int64_t>(nRollouts), feet, horizon, dT, rho,
+                      twists.planePointers(), positions.planePointers(), rotations.planePointers(),
+                      nullPoses.planePointers(), parameters ? parameters->planePointers() : nullptr,
+                      referenceWrench.data(), weights, gradCost, out(twistGradient), out(positionGradient),
+                      out(rotationGradient), out(nullPoseGradient), out(parameterGradient), stream),
+                  where);
 }
 
 bool ContactRolloutBatch::rollout(std::size_t nRollouts, int feet, int horizon, double dT, double rho,

@@ -96,6 +96,8 @@ struct blf_ccm_handle {
     unsigned tmap_next = 0;
     double* gen_work = nullptr;      // scratch of the general-size RLS kernel
     size_t gen_bytes = 0;
+    double* tape = nullptr;          // pose checkpoints of blf_ccm_rollout_cost_vjp (ordered as the rollout scratch)
+    size_t tape_bytes = 0;
     cudaEvent_t scratch_ev = nullptr;
     cudaStream_t scratch_stream = nullptr;   // stream of the last launch that used the scratch
     bool scratch_busy = false;
@@ -131,6 +133,7 @@ struct blf_ccm_handle {
     int tune_fbd_tile_kb = 0;    // BLF_CCM_TUNE_FBD_TILE_KB: shared-memory target per CTA of the floating-base Euler step (default 24)
     int tune_fbd_no_bulk = 0;    // BLF_CCM_TUNE_FBD_NO_BULK=1: floating-base Euler step with per-thread copies even when 16-byte aligned
     int tune_rls_pipe = 0;       // BLF_CCM_TUNE_RLS_PIPE=1: the plain one-estimator-per-thread RLS kernel instead of the pipelined one
+    int tune_vjp_seg = 0;        // BLF_CCM_TUNE_VJP_SEG=4: rollout-cost VJP with every group requested on 4-step tape segments (measurement aid)
     // peer-memory arg-min exchange
     int p2p_nranks = 0, p2p_rank = -1;
     bool p2p_connected = false;
@@ -241,6 +244,7 @@ extern "C" int blf_ccm_create(int device, blf_ccm_handle** out)
     h->tune_host_down = env_int("BLF_CCM_TUNE_HOST_DOWN");
     if (const char* v = getenv("BLF_CCM_TUNE_HOST_RAMP")) h->tune_host_ramp = atoi(v);
     h->tune_rls_pipe = env_int("BLF_CCM_TUNE_RLS_PIPE");
+    h->tune_vjp_seg = env_int("BLF_CCM_TUNE_VJP_SEG");
     h->tune_llt_general = env_int("BLF_CCM_TUNE_LLT_GENERAL");
     h->tune_rollout_chunk_mb = env_int("BLF_CCM_TUNE_ROLLOUT_CHUNK_MB");
     h->tune_no_rows = env_int("BLF_CCM_TUNE_NO_ROWS");
@@ -328,6 +332,7 @@ extern "C" int blf_ccm_destroy(blf_ccm_handle* h)
     if (h->counter) cudaFree(h->counter);
     if (h->partials) cudaFree(h->partials);
     if (h->gen_work) cudaFree(h->gen_work);
+    if (h->tape) cudaFree(h->tape);
     h->magic = 0;
     delete h;
     return BLF_CCM_OK;

@@ -124,6 +124,41 @@ __device__ __forceinline__ void kin_euler_step(Pose& s, const V3& v, const V3& w
     s.c2 = kin_col_step<BAUM>(s.c2, x2, k2, alpha, beta, dT);
 }
 
+// Reverse mode of kin_euler_step, fast_rcp(x) differentiated as 1/x.  With alpha = kin_alpha,
+// r = 1/det, beta = dT rho/2 r, k0 = c1 x c2, k1 = c2 x c0, k2 = c0 x c1, det = c0.k0:
+//   c_j' = alpha c_j + dT w x c_j + beta k_j,  p' = p + dT v.
+// On entry g holds the adjoint of the pose AFTER the step; on return the adjoint of the pose s before
+// it, and gv, gw the step's contribution to the twist's adjoint (only formed when TW):
+//   gv = dT p'bar     gw = dT sum_j c_j x c_j'bar     c_jbar = alpha c_j'bar + dT c_j'bar x w
+//   k_jbar = beta c_j'bar,  betabar = sum_j c_j'bar.k_j,  detbar = -betabar beta r,  c_jbar += detbar k_j
+//   and the cross products' adjoints: k0 feeds c1 (c2 x k0bar) and c2 (k0bar x c1), and so on.
+// Without the Baumgarte term only the first three lines remain, with alpha = 1.
+template <bool BAUM, bool TW>
+__device__ __forceinline__ void kin_euler_step_vjp(const Pose& s, const V3& w, double half_rho, double dT,
+                                                   Pose& g, V3& gv, V3& gw)
+{
+    const V3 b0 = g.c0, b1 = g.c1, b2 = g.c2;   // adjoints of the columns after the step
+    if constexpr (TW) {
+        gv = dT * g.p;
+        gw = dT * (cross(s.c0, b0) + cross(s.c1, b1) + cross(s.c2, b2));
+    }
+    double alpha = 1.0;
+    if constexpr (BAUM) alpha = kin_alpha(dT, half_rho);
+    g.c0 = alpha * b0 + dT * cross(b0, w);
+    g.c1 = alpha * b1 + dT * cross(b1, w);
+    g.c2 = alpha * b2 + dT * cross(b2, w);
+    if constexpr (BAUM) {
+        const V3 k0 = cross(s.c1, s.c2), k1 = cross(s.c2, s.c0), k2 = cross(s.c0, s.c1);
+        const double r = fast_rcp(dot3(s.c0, k0));
+        const double beta = __dmul_rn(kin_dthr(dT, half_rho), r);
+        const double gdet = -(dot3(b0, k0) + dot3(b1, k1) + dot3(b2, k2)) * beta * r;
+        const V3 q0 = beta * b0, q1 = beta * b1, q2 = beta * b2;   // adjoints of k0, k1, k2
+        g.c0 = g.c0 + gdet * k0 + cross(q1, s.c2) + cross(s.c1, q2);
+        g.c1 = g.c1 + gdet * k1 + cross(s.c2, q0) + cross(q2, s.c0);
+        g.c2 = g.c2 + gdet * k2 + cross(q0, s.c1) + cross(s.c0, q1);
+    }
+}
+
 struct KinArgs {
     const double* tw[6];
     double* pos[3];   // in/out
@@ -391,6 +426,242 @@ ccm_rollout_kernel(const __grid_constant__ RolloutArgs a)
     ptx::cp_async_wait<0>();
     if constexpr ((OUT & M_CTRL) != 0) {
         if (staged && a.ctrl_bulk && lane == 0) ptx::bulk_wait_read_all();
+    }
+}
+
+// ------------------------------------------------------------------------------------------------
+// Reverse mode of the fused rollout's cost (blf_ccm_rollout_cost_vjp): for cotangents gbar[r] of
+// cost[r], gbar^T dcost/d(twists, initial pose, null pose, parameters).  One lane per chain, one
+// 32-chain tile per warp, as ccm_rollout_kernel.
+//   forward   the pose recurrence alone (no wrench), twists through a per-lane cp.async ring S steps
+//             deep; the pose before every step t = kS (k < last segment) goes to the tape
+//             ([k][12][chains], time-major, coalesced); the last segment's pose stays in registers
+//             and its twists in the ring.
+//   reverse   segment by segment from the last: the segment's poses are recomputed from its
+//             checkpoint with kin_euler_step (bit-identical to the forward rollout) into shared
+//             memory, then t = end .. start: wrench at (twist_t, pose_t), cotangent
+//             (gF, gT) = 2 gbar (wf (F - Fref), wt (T - Tref)), the pose adjoint back through Euler
+//             step t (kin_euler_step_vjp; step H-1 does not enter the cost), plus vjp_wrench at step
+//             t; the twist gradient of step t is written.  Null-pose and parameter adjoints add up
+//             in registers; after t = 0 the pose adjoint is the initial pose's gradient.
+// The previous segment's twists are staged while this one is walked: slot sigma_k(j) holds step
+// kS + j, with sigma alternating between j and S-1-j from segment to segment, so the slot a step
+// frees during the backward walk is the one the previous segment's forward recompute needs next.
+// Accumulations are rounded on their own (__dadd_rn): vjp_wrench's products are never contracted
+// into them, so at H = 1 the result is blf_ccm_wrench_vjp_soa's, bit for bit.
+// ------------------------------------------------------------------------------------------------
+
+constexpr int kVjpSeg = 8;   // steps per tape segment (measured: profiles/r05_rollout_vjp_probe.log)
+
+struct RolloutVjpArgs {
+    const double* tw[6];      // [horizon*chains], index t*chains + chain
+    const double* pos0[3];    // [chains]
+    const double* rot0[9];
+    const double* nul[12];
+    const double* prm[4];     // per-chain parameters (HET)
+    const double* gcost;      // [n_rollouts]
+    double* gtw[6];           // [horizon*chains]   (G_TWIST)
+    double* gpos[3];          // [chains]           (G_POSE)
+    double* grot[9];
+    double* gnul[12];         // [chains]           (G_NULL)
+    double* gprm[4];          // [chains]           (G_PARAMS)
+    double* tape;             // [segments-1][12][chains]
+    double uni[4];            // uniform length, width, spring, damper
+    double ref[6];
+    double wf, wt;
+    double half_rho, dT;
+    long long chains;
+    int horizon;
+    int feet;
+};
+
+__device__ __forceinline__ V3 add_rn(const V3& a, const V3& b)
+{
+    return V3{__dadd_rn(a.x, b.x), __dadd_rn(a.y, b.y), __dadd_rn(a.z, b.z)};
+}
+
+template <bool HET, bool BAUM, unsigned GROUPS, int S>
+__global__ void __launch_bounds__(32)
+ccm_rollout_vjp_kernel(const __grid_constant__ RolloutVjpArgs a)
+{
+    static_assert(S >= 2 && (S & (S - 1)) == 0, "segment length: a power of two");
+    constexpr bool kTw = (GROUPS & G_TWIST) != 0;
+    constexpr bool kAdj = (GROUPS & (G_TWIST | G_POSE)) != 0;   // the pose adjoint recurrence is needed
+    constexpr unsigned W = GROUPS | (kAdj ? G_POSE : 0u);         // groups of the per-step wrench VJP
+    extern __shared__ __align__(128) unsigned char smem_raw[];
+
+    const int lane = threadIdx.x & 31;
+    const long long c = static_cast<long long>(blockIdx.x) * kWarp + lane;
+    if (c >= a.chains) return;   // no warp-collective operation below: idle lanes leave
+    const long long N = a.chains;
+    const int H = a.horizon;
+
+    double* ring = reinterpret_cast<double*>(smem_raw);   // [S][6][32] twists
+    double* poses = ring + S * 6 * kWarp;                 // [S][12][32] the segment's poses
+    const uint32_t ring_s = ptx::smem_addr(ring) + static_cast<uint32_t>(lane) * 8u;
+    auto stage = [&](int t, int slot) {
+        const uint32_t dst = ring_s + static_cast<uint32_t>(slot * 6 * kWarp * 8);
+        const long long src = static_cast<long long>(t) * N + c;
+#pragma unroll
+        for (int j = 0; j < 6; ++j) ptx::cp_async8(dst + j * kWarp * 8, a.tw[j] + src);
+    };
+    auto twist = [&](int slot, V3& v, V3& w) {
+        const double* r = ring + slot * 6 * kWarp + lane;
+        v = V3{r[0], r[kWarp], r[2 * kWarp]};
+        w = V3{r[3 * kWarp], r[4 * kWarp], r[5 * kWarp]};
+    };
+    // plain launch: as ccm_rollout_kernel (latency-bound, PDL measured worse there)
+#pragma unroll
+    for (int t = 0; t < S; ++t) {
+        if (t < H) stage(t, t);
+        ptx::cp_async_commit();
+    }
+
+    Pose s;
+    s.p = V3{__ldg(a.pos0[0] + c), __ldg(a.pos0[1] + c), __ldg(a.pos0[2] + c)};
+    s.c0 = V3{__ldg(a.rot0[0] + c), __ldg(a.rot0[3] + c), __ldg(a.rot0[6] + c)};
+    s.c1 = V3{__ldg(a.rot0[1] + c), __ldg(a.rot0[4] + c), __ldg(a.rot0[7] + c)};
+    s.c2 = V3{__ldg(a.rot0[2] + c), __ldg(a.rot0[5] + c), __ldg(a.rot0[8] + c)};
+    const V3 p0{__ldg(a.nul[0] + c), __ldg(a.nul[1] + c), __ldg(a.nul[2] + c)};
+    const V3 n1{__ldg(a.nul[3] + c), __ldg(a.nul[6] + c), __ldg(a.nul[9] + c)};
+    const V3 n2{__ldg(a.nul[4] + c), __ldg(a.nul[7] + c), __ldg(a.nul[10] + c)};
+    double len = a.uni[0], wid = a.uni[1], spr = a.uni[2], dmp = a.uni[3];
+    if constexpr (HET) {
+        len = __ldg(a.prm[0] + c); wid = __ldg(a.prm[1] + c);
+        spr = __ldg(a.prm[2] + c); dmp = __ldg(a.prm[3] + c);
+    }
+    const Prm q = make_prm(len, wid, spr, dmp);
+    const double g2 = 2.0 * __ldg(a.gcost + c / a.feet);
+    const double sF = g2 * a.wf, sT = g2 * a.wt;
+
+    // ---- forward sweep: poses of the segment starts
+    const int nseg = (H + S - 1) / S;
+    const int tl = (nseg - 1) * S;   // first step of the last segment
+    for (int t = 0; t < tl; ++t) {
+        if ((t & (S - 1)) == 0) {
+            double* k = a.tape + static_cast<long long>(t / S) * 12 * N + c;
+            __stcg(k, s.p.x); __stcg(k + N, s.p.y); __stcg(k + 2 * N, s.p.z);
+            __stcg(k + 3 * N, s.c0.x); __stcg(k + 4 * N, s.c0.y); __stcg(k + 5 * N, s.c0.z);
+            __stcg(k + 6 * N, s.c1.x); __stcg(k + 7 * N, s.c1.y); __stcg(k + 8 * N, s.c1.z);
+            __stcg(k + 9 * N, s.c2.x); __stcg(k + 10 * N, s.c2.y); __stcg(k + 11 * N, s.c2.z);
+        }
+        ptx::cp_async_wait<S - 1>();
+        V3 v, w;
+        twist(t & (S - 1), v, w);
+        kin_euler_step<BAUM>(s, v, w, a.half_rho, a.dT);
+        if (t + S < H) stage(t + S, (t + S) & (S - 1));   // the slot just consumed
+        ptx::cp_async_commit();
+    }
+    // the ring now holds the last segment, step tl + j in slot j
+
+    // ---- reverse sweep
+    Pose gs{};               // adjoint of the pose
+    V3 gp0{}, gn1{}, gn2{};  // null pose
+    double gL = 0.0, gW = 0.0, gk = 0.0, gb = 0.0;
+    const V3 rf{a.ref[0], a.ref[1], a.ref[2]}, rt{a.ref[3], a.ref[4], a.ref[5]};
+    int flip = 0;            // sigma_k(j) = flip ? S-1-j : j
+    for (int k = nseg - 1; k >= 0; --k) {
+        const int t0 = k * S;
+        const int n = min(S, H - t0);
+        ptx::cp_async_wait<0>();
+        if (k != nseg - 1) {
+            const double* ck = a.tape + static_cast<long long>(k) * 12 * N + c;
+            s.p = V3{__ldcg(ck), __ldcg(ck + N), __ldcg(ck + 2 * N)};
+            s.c0 = V3{__ldcg(ck + 3 * N), __ldcg(ck + 4 * N), __ldcg(ck + 5 * N)};
+            s.c1 = V3{__ldcg(ck + 6 * N), __ldcg(ck + 7 * N), __ldcg(ck + 8 * N)};
+            s.c2 = V3{__ldcg(ck + 9 * N), __ldcg(ck + 10 * N), __ldcg(ck + 11 * N)};
+        }
+        for (int j = 0; j < n; ++j) {
+            double* o = poses + j * 12 * kWarp + lane;
+            o[0] = s.p.x; o[kWarp] = s.p.y; o[2 * kWarp] = s.p.z;
+            o[3 * kWarp] = s.c0.x; o[4 * kWarp] = s.c0.y; o[5 * kWarp] = s.c0.z;
+            o[6 * kWarp] = s.c1.x; o[7 * kWarp] = s.c1.y; o[8 * kWarp] = s.c1.z;
+            o[9 * kWarp] = s.c2.x; o[10 * kWarp] = s.c2.y; o[11 * kWarp] = s.c2.z;
+            if (j + 1 < n) {
+                V3 v, w;
+                twist(flip ? S - 1 - j : j, v, w);
+                kin_euler_step<BAUM>(s, v, w, a.half_rho, a.dT);
+            }
+        }
+        // slot sigma_k(j) takes step (k-1)S + S-1-j of the previous segment once step kS + j is done;
+        // the slots this (last, short) segment does not use take theirs now
+        if (k > 0)
+            for (int j = n; j < S; ++j) stage(t0 - 1 - j, flip ? S - 1 - j : j);
+        for (int j = n - 1; j >= 0; --j) {
+            const int t = t0 + j;
+            const int slot = flip ? S - 1 - j : j;
+            V3 v, w;
+            twist(slot, v, w);
+            if (k > 0) stage(t0 - 1 - j, slot);
+            const double* o = poses + j * 12 * kWarp + lane;
+            Pose ps;
+            ps.p = V3{o[0], o[kWarp], o[2 * kWarp]};
+            ps.c0 = V3{o[3 * kWarp], o[4 * kWarp], o[5 * kWarp]};
+            ps.c1 = V3{o[6 * kWarp], o[7 * kWarp], o[8 * kWarp]};
+            ps.c2 = V3{o[9 * kWarp], o[10 * kWarp], o[11 * kWarp]};
+
+            State st;
+            st.v = v; st.w = w; st.p = ps.p; st.p0 = p0;
+            st.e1 = ps.c0; st.e2 = ps.c1;
+            st.R02 = ps.c2.x; st.R12 = ps.c2.y; st.R22 = ps.c2.z;
+            st.n1 = n1; st.n2 = n2;
+            Result r;
+            eval_contact<M_WRENCH>(st, q, r);
+            const V3 gF = sF * (r.force - rf), gT = sT * (r.torque - rt);
+            VjpOut g;
+            vjp_wrench<W>(st, q, len, wid, gF, gT, g);
+
+            const bool last = t == H - 1;   // the step after it does not enter the cost
+            V3 gv{}, gw{};
+            if constexpr (kTw) gv = g.v, gw = g.w;
+            if constexpr (kAdj) {
+                if (last) {
+                    gs.p = g.p;
+                    gs.c0 = g.e1;
+                    gs.c1 = g.e2;
+                    gs.c2 = V3{0.0, 0.0, g.R22};
+                } else {
+                    V3 ev{}, ew{};
+                    kin_euler_step_vjp<BAUM, kTw>(ps, w, a.half_rho, a.dT, gs, ev, ew);
+                    if constexpr (kTw) gv = add_rn(ev, g.v), gw = add_rn(ew, g.w);
+                    gs.p = add_rn(gs.p, g.p);
+                    gs.c0 = add_rn(gs.c0, g.e1);
+                    gs.c1 = add_rn(gs.c1, g.e2);
+                    gs.c2.z = __dadd_rn(gs.c2.z, g.R22);
+                }
+            }
+            if constexpr (kTw) {
+                const long long i = static_cast<long long>(t) * N + c;
+                __stcs(a.gtw[0] + i, gv.x); __stcs(a.gtw[1] + i, gv.y); __stcs(a.gtw[2] + i, gv.z);
+                __stcs(a.gtw[3] + i, gw.x); __stcs(a.gtw[4] + i, gw.y); __stcs(a.gtw[5] + i, gw.z);
+            }
+            if constexpr ((GROUPS & G_NULL) != 0) {
+                if (last) gp0 = g.p0, gn1 = g.n1, gn2 = g.n2;
+                else gp0 = add_rn(gp0, g.p0), gn1 = add_rn(gn1, g.n1), gn2 = add_rn(gn2, g.n2);
+            }
+            if constexpr ((GROUPS & G_PARAMS) != 0) {
+                if (last) gL = g.L, gW = g.W, gk = g.k, gb = g.b;
+                else gL = __dadd_rn(gL, g.L), gW = __dadd_rn(gW, g.W), gk = __dadd_rn(gk, g.k), gb = __dadd_rn(gb, g.b);
+            }
+        }
+        ptx::cp_async_commit();
+        flip ^= 1;
+    }
+
+    if constexpr ((GROUPS & G_POSE) != 0) {
+        a.gpos[0][c] = gs.p.x; a.gpos[1][c] = gs.p.y; a.gpos[2][c] = gs.p.z;
+        a.grot[0][c] = gs.c0.x; a.grot[1][c] = gs.c1.x; a.grot[2][c] = gs.c2.x;
+        a.grot[3][c] = gs.c0.y; a.grot[4][c] = gs.c1.y; a.grot[5][c] = gs.c2.y;
+        a.grot[6][c] = gs.c0.z; a.grot[7][c] = gs.c1.z; a.grot[8][c] = gs.c2.z;
+    }
+    if constexpr ((GROUPS & G_NULL) != 0) {
+        a.gnul[0][c] = gp0.x; a.gnul[1][c] = gp0.y; a.gnul[2][c] = gp0.z;
+        a.gnul[3][c] = gn1.x; a.gnul[4][c] = gn2.x; a.gnul[5][c] = 0.0;
+        a.gnul[6][c] = gn1.y; a.gnul[7][c] = gn2.y; a.gnul[8][c] = 0.0;
+        a.gnul[9][c] = gn1.z; a.gnul[10][c] = gn2.z; a.gnul[11][c] = 0.0;
+    }
+    if constexpr ((GROUPS & G_PARAMS) != 0) {
+        a.gprm[0][c] = gL; a.gprm[1][c] = gW; a.gprm[2][c] = gk; a.gprm[3][c] = gb;
     }
 }
 

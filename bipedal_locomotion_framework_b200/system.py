@@ -179,6 +179,45 @@ class KinematicsBatch:
         return call
 
 
+# gradient groups of blf_ccm_rollout_cost_vjp and the output planes of each
+ROLLOUT_VJP_GROUPS = {"twist": ("twist",), "pose": ("pos", "rot"), "null": ("null",), "params": ("params",)}
+
+_ROLLOUT_COST_FN = None
+
+
+def _rollout_cost_function():
+    """torch.autograd.Function of RolloutBatch.rollout_cost (built on first use, so importing this
+    module does not import torch)."""
+    global _ROLLOUT_COST_FN
+    if _ROLLOUT_COST_FN is not None:
+        return _ROLLOUT_COST_FN
+    import torch
+    from torch.autograd.function import once_differentiable
+
+    class RolloutCost(torch.autograd.Function):
+        @staticmethod
+        def forward(ctx, rb, cfg, twist, pos, rot, null, params):
+            ctx.rb, ctx.cfg = rb, cfg
+            ctx.save_for_backward(twist, pos, rot, null, params)
+            return rb.run(*cfg[:5], twist, pos, rot, null, *cfg[5:], param_planes=params)["cost"]
+
+        @staticmethod
+        @once_differentiable
+        def backward(ctx, grad_cost):
+            twist, pos, rot, null, params = ctx.saved_tensors
+            need = dict(zip(("twist", "pos", "rot", "null", "params"), ctx.needs_input_grad[2:]))
+            groups = {g for g, keys in ROLLOUT_VJP_GROUPS.items() if any(need[k] for k in keys)}
+            if not groups:
+                return (None,) * 7
+            g = ctx.rb.cost_vjp(*ctx.cfg[:5], twist, pos, rot, null, *ctx.cfg[5:], grad_cost.contiguous(),
+                                param_planes=params, inputs=groups)
+            return (None, None) + tuple(g.get(k) if need[k] else None
+                                        for k in ("twist", "pos", "rot", "null", "params"))
+
+    _ROLLOUT_COST_FN = RolloutCost
+    return RolloutCost
+
+
 class RolloutBatch:
     """Fused sampling-MPC rollouts (blf_ccm_rollout_integrate_cost) on one GPU."""
 
@@ -229,6 +268,70 @@ class RolloutBatch:
         call, out = self.prepare(*args, **kw)
         call()
         return out
+
+    def _vjp_args(self, n_rollouts, feet, horizon, dT, rho, twist_planes, pos_planes, rot_planes,
+                  null_planes, wrench_ref, weights, grad_cost, param_planes, inputs, out):
+        """Arguments of blf_ccm_rollout_cost_vjp and the output dict (see cost_vjp)."""
+        t = self._torch
+        chains = n_rollouts * feet
+        groups = set(ROLLOUT_VJP_GROUPS) if inputs is True else set(inputs or ())
+        assert groups <= set(ROLLOUT_VJP_GROUPS), f"unknown gradient groups {groups - set(ROLLOUT_VJP_GROUPS)}"
+        if out is None:
+            mk = lambda *s: t.empty(s, dtype=t.float64, device=self.device)
+            shapes = {"twist": (6, horizon * chains), "pos": (3, chains), "rot": (9, chains),
+                      "null": (12, chains), "params": (4, chains)}
+            out = {k: mk(*shapes[k]) for g in groups for k in ROLLOUT_VJP_GROUPS[g]}
+        ref = np.ascontiguousarray(wrench_ref, dtype=np.float64)
+        wts = np.ascontiguousarray(weights, dtype=np.float64)
+        pp = ContinuousContactModelBatch._plane_ptrs
+        args = (self._b.handle.ptr, int(n_rollouts), int(feet), int(horizon), float(dT), float(rho),
+                pp(twist_planes, 6), pp(pos_planes, 3), pp(rot_planes, 9), pp(null_planes, 12),
+                pp(param_planes, 4), _np_ptr(ref), _np_ptr(wts), grad_cost.data_ptr(),
+                pp(out.get("twist"), 6), pp(out.get("pos"), 3), pp(out.get("rot"), 9),
+                pp(out.get("null"), 12), pp(out.get("params"), 4), self._b._stream())
+        keep = (twist_planes, pos_planes, rot_planes, null_planes, param_planes, grad_cost, out, ref, wts)
+        return args, out, keep
+
+    def cost_vjp(self, n_rollouts, feet, horizon, dT, rho, twist_planes, pos_planes, rot_planes,
+                 null_planes, wrench_ref, weights, grad_cost, param_planes=None, inputs=True,
+                 out: dict | None = None) -> dict:
+        """Reverse mode of the rollouts' cost (blf_ccm_rollout_cost_vjp): for the (n_rollouts,)
+        cotangent `grad_cost` of the cost `run` computes from the same arguments, returns
+        grad_cost^T dcost/d(input) for the requested groups only.  `inputs`: True for every group or
+        a subset of "twist", "pose", "null", "params"; the dict holds "twist" (6, horizon*chains),
+        "pos" (3, chains) and "rot" (9, chains) for "pose", "null" (12, chains) and "params"
+        (4, chains: each chain's contribution; with uniform parameters the sum is their gradient)."""
+        args, out, _ = self._vjp_args(n_rollouts, feet, horizon, dT, rho, twist_planes, pos_planes,
+                                      rot_planes, null_planes, wrench_ref, weights, grad_cost,
+                                      param_planes, inputs, out)
+        _capi.check(_capi.lib().blf_ccm_rollout_cost_vjp(*args))
+        return out
+
+    def prepare_cost_vjp(self, n_rollouts, feet, horizon, dT, rho, twist_planes, pos_planes,
+                         rot_planes, null_planes, wrench_ref, weights, grad_cost, param_planes=None,
+                         inputs=True, out: dict | None = None):
+        """Prepared form of cost_vjp (every argument bound once).  Returns (call, out)."""
+        args, out, keep = self._vjp_args(n_rollouts, feet, horizon, dT, rho, twist_planes, pos_planes,
+                                         rot_planes, null_planes, wrench_ref, weights, grad_cost,
+                                         param_planes, inputs, out)
+        fn = _capi.lib().blf_ccm_rollout_cost_vjp
+
+        def call(_keep=keep):
+            rc = fn(*args)
+            if rc:
+                _capi.check(rc)
+        return call, out
+
+    def rollout_cost(self, n_rollouts, feet, horizon, dT, rho, twist_planes, pos_planes, rot_planes,
+                     null_planes, wrench_ref, weights, param_planes=None):
+        """(n_rollouts,) cost of `run` through torch.autograd: gradients reach the twist (6,
+        horizon*chains), pos (3, chains), rot (9, chains), null (12, chains) and param (4, chains)
+        tensors that require them.  The backward is blf_ccm_rollout_cost_vjp, asked only for the
+        groups that need a gradient; it is not itself differentiable."""
+        cfg = (int(n_rollouts), int(feet), int(horizon), float(dT), float(rho),
+               np.array(wrench_ref, dtype=np.float64), np.array(weights, dtype=np.float64))
+        return _rollout_cost_function().apply(self, cfg, twist_planes, pos_planes, rot_planes,
+                                              null_planes, param_planes)
 
     def run_host(self, n_rollouts, feet, horizon, dT, rho, twist_planes, pos_planes, rot_planes,
                  null_planes, wrench_ref, weights, param_planes=None, want_cost: bool = True):

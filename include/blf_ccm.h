@@ -363,6 +363,35 @@ BLF_CCM_API int blf_ccm_rollout_integrate_cost(
     double* const* final_rot_planes, const double* host_wrench_ref, const double* host_weights,
     int64_t index_base, double* cost, void* best, void* stream);
 
+/*
+ * Reverse mode of blf_ccm_rollout_integrate_cost's cost (no reference counterpart computes it): for
+ * cotangents grad_cost[r] of cost[r], writes grad_cost^T dcost/d(twists, initial pose, null pose,
+ * length, width, spring, damper), the cost exactly as blf_ccm_rollout_integrate_cost defines it and
+ * the derivative that of the device's own forward arithmetic (the regrouped Baumgarte update, its
+ * reciprocal taken as 1/x; the derivative of |R22| at R22 = +-0 is taken as 0).
+ *   n_rollouts ... host_weights   as blf_ccm_rollout_integrate_cost (same planes, same layout)
+ *   grad_cost                   device, n_rollouts doubles; required
+ *   grad_twist_planes[6]        horizon*chains doubles each, index t*chains + c (time-major), or NULL
+ *   grad_pos_planes[3], grad_rot_planes[9]   the initial pose (row-major rotation), both or neither
+ *   grad_null_planes[12]        the null pose; its third rotation column (5, 8, 11) receives +0.0
+ *   grad_param_planes[4]        each chain's contribution to the gradient of length, width, spring,
+ *                               damper; with uniform parameters their sum is the shared values' gradient
+ * A non-NULL output array requests its group; every plane in it is written.  Outputs must not alias
+ * any input.  Nothing requested or grad_cost NULL, n_rollouts < 0, feet < 1 or horizon < 1 (with
+ * n_rollouts > 0), or a NULL / misaligned plane that is read or requested is BLF_CCM_ERR_INVALID_ARG
+ * (nothing is launched); n_rollouts = 0 is a no-op.  One launch.  The pose checkpoints
+ * (12 doubles per chain every 8 steps) live in the handle's rollout scratch, so this call is ordered
+ * with the rollout entry points like they are with one another.
+ */
+BLF_CCM_API int blf_ccm_rollout_cost_vjp(
+    blf_ccm_handle* h, int64_t n_rollouts, int feet, int horizon, double dT, double rho,
+    const double* const* twist_planes, const double* const* pos_planes,
+    const double* const* rot_planes, const double* const* null_planes,
+    const double* const* param_planes, const double* host_wrench_ref, const double* host_weights,
+    const double* grad_cost, double* const* grad_twist_planes, double* const* grad_pos_planes,
+    double* const* grad_rot_planes, double* const* grad_null_planes,
+    double* const* grad_param_planes, void* stream);
+
 /* Same rollouts with every plane in HOST memory (pinned gives full PCIe speed), cost only: the
  * horizon is cut into time chunks (contiguous in the time-major planes, so every upload is a plain
  * 1-D copy), pipelined through four slots -- the upload of the next chunk overlaps the kernel of
