@@ -163,6 +163,35 @@ def exact_eval_rounded(twist, pose, null_pose, params):
     return {k: np.array([float(x) for x in vals]) for k, vals in ex.items()}
 
 
+def exact_rollout_cost(states, rollout_len, wrench_ref, weights, params):
+    """Cost of each rollout of a rollout-major batch, cost[r] = sum_e wf|F_e - Fref|^2 +
+    wt|T_e - Tref|^2 over the exact wrenches of exact_eval, summed in Fraction and rounded once.
+
+    states: dict with twists (n, 6), poses (n, 12), null_poses (n, 12); params: (n, 4) per state, or
+    one (length, width, spring, damper) for all; n a multiple of rollout_len.  Repeated states are
+    evaluated once."""
+    tw, po, nu = (np.asarray(states[k], dtype=np.float64) for k in ("twists", "poses", "null_poses"))
+    n = tw.shape[0]
+    assert n % rollout_len == 0
+    prm = np.asarray(params, dtype=np.float64)
+    prm = np.broadcast_to(prm, (n, 4)) if prm.ndim == 1 else prm
+    ref = [F(float(x)) for x in wrench_ref]
+    wf, wt = F(float(weights[0])), F(float(weights[1]))
+    memo = {}
+
+    def contact_cost(i):
+        key = tw[i].tobytes() + po[i].tobytes() + nu[i].tobytes() + prm[i].tobytes()
+        if key not in memo:
+            w = exact_eval(tw[i], po[i], nu[i], prm[i])["wrench"]
+            qf = sum((w[c] - ref[c]) ** 2 for c in range(3))
+            qt = sum((w[3 + c] - ref[3 + c]) ** 2 for c in range(3))
+            memo[key] = wf * qf + wt * qt
+        return memo[key]
+
+    return np.array([float(sum((contact_cost(r * rollout_len + e) for e in range(rollout_len)), F(0)))
+                     for r in range(n // rollout_len)])
+
+
 def _edge_states():
     """Hand-picked states the random stream does not reach."""
     from bipedal_locomotion_framework_b200 import synthetic as syn
